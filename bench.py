@@ -2,6 +2,7 @@
 """bench.py — YOLO11 inference hot path on B200: preprocessed tensor in -> NMS'd detections out.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model n|s|m] [--batch B]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...       (one rank per GPU, weak scaling)
 
 One "step" = one pass of the hot path over one batch of synthetic 640x640 images (BASELINE.json config 3:
@@ -31,6 +32,7 @@ import threading
 import time
 from pathlib import Path
 
+import numpy as np
 import torch
 
 ROOT = Path(__file__).resolve().parent
@@ -57,7 +59,12 @@ def parse():
                     help="skip the secondary BASELINE configs (yolo11m bs=256 sharded, NMS stress, eager GPU baseline, H2D ceiling)")
     ap.add_argument("--inflight", type=int, default=2,
                     help="batches in flight per GPU (each on its own stream with its own plan buffers)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0's batch) as DIR/*.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 # ------------------------------------------------------------------------------------------------ synthetic
@@ -143,7 +150,8 @@ def cpu_reference_step(sd, x):
 
 def time_cpu(model_sd, batch, reps, warm=1, budget_s=None):
     """Median images/s of the CPU path on `batch`-image steps; with `budget_s` keep repeating (>= reps) until about
-    that much CPU wall time has been spent, so the baseline is a 10-30 s sample, not a single cold step."""
+    that much CPU wall time has been spent, so the baseline is a 10-30 s sample, not a single cold step.
+    Also returns the last step's detections (a list of (n, 6) arrays, one per image)."""
     x = synth_images(batch, 1, seed=0)[0]
     for _ in range(warm):
         cpu_reference_step(model_sd, x)
@@ -151,9 +159,24 @@ def time_cpu(model_sd, batch, reps, warm=1, budget_s=None):
     t_start = time.perf_counter()
     while len(ts) < reps or (budget_s is not None and time.perf_counter() - t_start < budget_s and len(ts) < 400):
         t0 = time.perf_counter()
-        cpu_reference_step(model_sd, x)
+        out = cpu_reference_step(model_sd, x)
         ts.append(time.perf_counter() - t0)
-    return batch / statistics.median(ts), ts
+    return batch / statistics.median(ts), ts, out
+
+
+def dump_outputs(out_dir, dets, counts, limit_bytes=64 << 20):
+    """Write one step's result as `out_dir`/dets.npy ((B, MAX_DET, 6) float32: x1, y1, x2, y2, conf, class) and
+    counts.npy ((B,) float64).  Rows at or past an image's count are not part of the result (the GPU path leaves
+    them unwritten), so they are stored as zeros and two builds compare equal exactly when their detections do.
+    A batch too large for `limit_bytes` is cut to its first images."""
+    keep = max(1, limit_bytes // (MAX_DET * 6 * 4 + 8))
+    dets = np.array(dets[:keep], dtype=np.float32)
+    counts = np.asarray(counts[:keep], dtype=np.int64)
+    dets[np.arange(MAX_DET)[None, :] >= counts[:, None]] = 0
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "dets.npy", dets)
+    np.save(out / "counts.npy", counts.astype(np.float64))
 
 
 def ncu_traffic(kernel, model_name, batch):
@@ -381,10 +404,14 @@ def main():
         t_probe0 = time.perf_counter()
         cpu_reference_step(sd, synth_images(sample_b, 1)[0])
         probe = time.perf_counter() - t_probe0
-        budget = 150.0                                      # keep the whole arm within a few minutes
-        steps = max(1, min(a.steps, int(budget / max(probe, 1e-3)) - a.warmup))
+        steps = a.steps
         warm = min(a.warmup, max(0, int(20.0 / max(probe, 1e-3))))
-        v, ts = time_cpu(sd, sample_b, steps, warm)
+        v, ts, last = time_cpu(sd, sample_b, steps, warm)
+        if a.dump_outputs:
+            dets = np.zeros((sample_b, MAX_DET, 6), np.float32)
+            for i, d in enumerate(last):
+                dets[i, :len(d)] = d
+            dump_outputs(a.dump_outputs, dets, [len(d) for d in last])
         line = {
             "impl": "reference", "metric": "images_per_sec", "value": round(v, 3), "unit": "images/s",
             "n_gpus": a.gpus, "steps": steps, "warmup": warm, "ms_per_step": round(statistics.median(ts) * 1e3, 3),
@@ -478,6 +505,9 @@ def main():
         for _ in range(max(1, a.repeats)):
             ms_r, (dets, counts) = timed(a.steps, n_fly)
             rep_ms.append(ms_r)
+        if a.dump_outputs and rank == 0:
+            # the returned tensors alias plan buffers that the steps below overwrite: copy the last timed step now
+            dump_outputs(a.dump_outputs, dets.cpu().numpy(), counts.cpu().numpy())
         ms_max = statistics.median(rep_ms)
         ms_serial = ms_max
         if n_fly > 1:
@@ -589,8 +619,6 @@ def main():
     # ---- image preprocess (SURVEY §8f rank 1): uint8 HWC BGR images -> letterboxed fp32 NCHW batch on the GPU
     prep = None
     if rank == 0 and not a.no_e2e:
-        import numpy as np
-
         from yololite.data import letterbox_batch_cuda
         from yololite.data.augment import _Staging
 
@@ -693,7 +721,7 @@ def main():
             os.sched_setaffinity(0, numa[0])            # the CPU baseline may use every host core again
         threads = max(1, min(os.cpu_count() or 1, 64))
         torch.set_num_threads(threads)
-        v, ts = time_cpu(sd_cpu, 8, reps=3, warm=1, budget_s=12.0)
+        v, ts, _ = time_cpu(sd_cpu, 8, reps=3, warm=1, budget_s=12.0)
         cpu_b = {"value": round(v, 3), "unit": "images/s", "cores": threads, "kind": "port",
                  "sample": f"oracle port (yolo11_ref fp32 unfused + nms_ref), 8-image steps of the bs={a.batch} "
                            f"workload x{len(ts)} reps, {sum(ts):.1f}s CPU wall, median step"}
