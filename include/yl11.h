@@ -336,6 +336,36 @@ typedef struct yl_lb_image {
  * imgs_dev: n descriptors in DEVICE memory. */
 int yl_letterbox_u8(const yl_lb_image* imgs_dev, int n, float* dst_nchw, int H, int W, int pad_value, void* stream);
 
+/* ---- test-time augmentation (DetectionModel._predict_augment, nn/tasks.py) -------------------------------------- */
+/* One augmented input of _predict_augment: scale_img(x.flip(3) if flip else x, ratio, gs) (utils/torch_utils.py), i.e.
+ * F.interpolate(bilinear, align_corners=False) to the content size (h, w) at the top-left of an (H, W) canvas whose other
+ * pixels are F.pad's 0.447.  y: dense (n, c, H, W) fp32, 16-byte aligned, W % 4 == 0. */
+typedef struct yl_tta_canvas {
+    float* y;
+    int32_t H, W;    /* canvas */
+    int32_t h, w;    /* resized content (int(h * ratio), int(w * ratio)) */
+    int32_t flip;    /* 1: left-right flip before the resize */
+    int32_t _pad;
+} yl_tta_canvas;
+/* The scale_img calls of passes 1 and 2 of _predict_augment in ONE launch: x is the (n, c, h, w) batch in YL_F32,
+ * YL_F16 (widened) or YL_U8 (value / 255 in fp32, the model input after the predictor's `/255`), read once for both
+ * canvases[2].  Same arithmetic as ATen's upsample_bilinear2d; w <= 6144. */
+int yl_tta_scale_img(const void* x, int x_dtype, int n, int c, int h, int w, const yl_tta_canvas* canvases, void* stream);
+/* One pass of _predict_augment as seen by the merge: its prediction (B, 4+nc, A) fp32 and the anchors [a0, a0+n) that
+ * _clip_augmented keeps. */
+typedef struct yl_tta_pass {
+    const float* pred;
+    int32_t A;
+    int32_t a0, n;
+    int32_t flip;    /* 1: left-right flip (flips == 3 of _descale_pred) */
+    float scale;     /* the pass's scale_img ratio */
+    int32_t _pad;
+} yl_tta_pass;
+/* _descale_pred + _clip_augmented + torch.cat(y, -1) of _predict_augment over passes[3]: y (B, 4+nc, sum n) fp32 gets,
+ * per pass in order, its kept anchors with rows 0..3 multiplied by the fp32 reciprocal of `scale` (torch's CUDA
+ * `p[:, :4] /= scale`) and, for a flipped pass, row 0 replaced by img_w - x.  Bit-identical to those torch ops on CUDA. */
+int yl_tta_merge(const yl_tta_pass* passes, int B, int nc, int img_w, float* y, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

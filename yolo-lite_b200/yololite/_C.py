@@ -112,6 +112,19 @@ class ConvChain(C.Structure):
                                                                    "tmem_cols", "reserved")]
 
 
+class TtaCanvas(C.Structure):
+    """Mirror of `yl_tta_canvas` (32 bytes)."""
+
+    _fields_ = [("y", C.c_void_p)] + [(k, C.c_int32) for k in ("H", "W", "h", "w", "flip", "_pad")]
+
+
+class TtaPass(C.Structure):
+    """Mirror of `yl_tta_pass` (32 bytes)."""
+
+    _fields_ = [("pred", C.c_void_p), ("A", C.c_int32), ("a0", C.c_int32), ("n", C.c_int32), ("flip", C.c_int32),
+                ("scale", C.c_float), ("_pad", C.c_int32)]
+
+
 _PROTOTYPES = {
     "yl_version": (C.c_int, []),
     "yl_last_error_string": (C.c_char_p, []),
@@ -173,6 +186,9 @@ _PROTOTYPES = {
     "yl_match_predictions": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                        C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "yl_letterbox_u8": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "yl_tta_scale_img": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(TtaCanvas),
+                                   C.c_void_p]),
+    "yl_tta_merge": (C.c_int, [C.POINTER(TtaPass), C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
 }
 
 EXPORTS = tuple(_PROTOTYPES)

@@ -239,7 +239,8 @@ class NmsWorkspace:
 
 def nms_batched(pred: torch.Tensor, conf: float, iou: float, classes=None, agnostic=False, multi_label=False,
                 max_det=300, max_nms=30000, max_wh=7680.0, out=None, counts=None):
-    """pred (B, 4+nc, A) fp32 contiguous CUDA -> (dets (B, max_det, 6) fp32, counts (B,) int32), all async."""
+    """pred (B, 4+nc, A) fp32 contiguous CUDA -> (dets (B, max_det, 6) fp32, counts (B,) int32), all async.
+    `classes`: None, a sequence of class ids, or a contiguous int32 tensor of them on pred's device."""
     lib = _C.init(pred.device)
     assert pred.is_cuda and pred.dtype == torch.float32 and pred.is_contiguous() and pred.dim() == 3
     B, C4, A = pred.shape
@@ -251,7 +252,9 @@ def nms_batched(pred: torch.Tensor, conf: float, iou: float, classes=None, agnos
     if counts is None:
         counts = torch.empty((B,), dtype=torch.int32, device=pred.device)
     cls_t = None
-    if classes is not None:
+    if isinstance(classes, torch.Tensor):   # already a device int32 list: no host->device copy (and no sync) per call
+        cls_t = classes
+    elif classes is not None:
         cls_t = torch.as_tensor(list(classes), dtype=torch.int32).to(pred.device)
     _C.check(lib.yl_nms_batched(pred.data_ptr(), B, nc, A, float(conf), float(iou), _ptr(cls_t),
                                 0 if cls_t is None else cls_t.numel(), int(agnostic), int(multi_label), int(max_det),
@@ -272,3 +275,23 @@ def nms_boxes(boxes: torch.Tensor, scores: torch.Tensor, iou: float) -> torch.Te
     _C.check(lib.yl_nms_boxes(boxes.data_ptr(), scores.data_ptr(), n, float(iou), ws.data_ptr(), ws.numel(),
                               keep.data_ptr(), count.data_ptr(), _C.stream_ptr()), "yl_nms_boxes")
     return keep[: int(count.item())]
+
+
+def tta_scale_img(x: torch.Tensor, canvases):
+    """scale_img of test-time augmentation passes 1 and 2 in one launch (yl_tta_scale_img).  x: contiguous (n, c, h, w)
+    CUDA batch, fp32 / fp16 / uint8 image bytes; canvases: two (y (n, c, H, W) fp32, (h_content, w_content), flip)."""
+    n, c, h, w = x.shape
+    arr = (_C.TtaCanvas * 2)(*[_C.TtaCanvas(y.data_ptr(), y.shape[2], y.shape[3], ch, cw, int(bool(flip)), 0)
+                               for y, (ch, cw), flip in canvases])
+    _C.check(_C.load().yl_tta_scale_img(x.data_ptr(), _C.INGEST_DTYPES[x.dtype], n, c, h, w, arr, _C.stream_ptr()),
+             "yl_tta_scale_img")
+
+
+def tta_merge(passes, img_w: int, out: torch.Tensor) -> torch.Tensor:
+    """_descale_pred + _clip_augmented + cat of the three passes (yl_tta_merge).  passes: three (pred (B, 4+nc, A) fp32,
+    first kept anchor, kept count, scale, flip); out: (B, 4+nc, sum of kept counts) fp32."""
+    B, C4, _ = out.shape
+    arr = (_C.TtaPass * 3)(*[_C.TtaPass(p.data_ptr(), p.shape[2], a0, n, int(bool(flip)), float(s), 0)
+                             for p, a0, n, s, flip in passes])
+    _C.check(_C.load().yl_tta_merge(arr, B, C4 - 4, int(img_w), out.data_ptr(), _C.stream_ptr()), "yl_tta_merge")
+    return out

@@ -188,7 +188,7 @@ class DetectionPredictor:
                 # model + NMS of the chunk are one CUDA-graph launch; its plan-owned outputs are gathered into the
                 # batch-level buffers (115 KB per 16 images)
                 d, c = model.infer_nms(buf[k * cb:(k + 1) * cb], a.conf, a.iou, a.classes, a.agnostic_nms, False,
-                                       a.max_det, slot=li)
+                                       a.max_det, slot=li, augment=a.augment)
                 if pipe["snap"] is not None:
                     ln.wait_event(pipe["snap"])  # the previous call's snapshot of the batch-level dets / counts is taken
                 st["dets"][k * cb:(k + 1) * cb].copy_(d, non_blocking=True)
@@ -291,7 +291,8 @@ class DetectionPredictor:
                         im = self.preprocess(im0s)
                     with profilers[1]:
                         a = self.args
-                        nms_out = self.model.model.infer_nms(im, a.conf, a.iou, a.classes, a.agnostic_nms, False, a.max_det)
+                        nms_out = self.model.model.infer_nms(im, a.conf, a.iou, a.classes, a.agnostic_nms, False, a.max_det,
+                                                             augment=a.augment)
                     with profilers[2]:
                         self.results = self.postprocess(None, im, im0s, nms_out=nms_out)
                 n = len(self.results)

@@ -135,7 +135,7 @@ class DetectionValidator:
         self.init_metrics(model)
         for batch in self.dataloader:
             batch = self.preprocess(batch)
-            y, _ = model.infer(batch["img"])
+            y, _ = model.infer(batch["img"], augment=self.args.augment)
             preds = self.postprocess(y)
             self.update_metrics(preds, batch)
         stats = self.get_stats()

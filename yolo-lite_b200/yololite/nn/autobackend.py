@@ -45,10 +45,11 @@ class AutoBackend(nn.Module):
         self.batch = batch
 
     def forward(self, im, augment=False, visualize=False, embed=None):
-        if augment or visualize or embed:
-            raise NotImplementedError("augment / visualize / embed are not part of the inference hot path")
-        y, raws = self.model.infer(im)
-        return [y, raws]
+        """[y, raw maps]; with `augment=True` [merged test-time-augmentation prediction, None]."""
+        if visualize or embed:
+            raise NotImplementedError("visualize / embed are not part of the inference hot path")
+        y, raws = self.model.infer(im, augment=augment)
+        return [y, None] if augment else [y, raws]
 
     def warmup(self, imgsz=(1, 3, 640, 640)):
         """Build (and graph-capture) the plan for `imgsz` ahead of the first real batch."""

@@ -6,7 +6,9 @@ Public surface follows reference yololite/nn/tasks.py: `DetectionModel(cfg, ch, 
 `attempt_load_one_weight / attempt_load_weights` (:461-522).  The layer loop of `_predict_once` (:118-145)
 exists only at plan-build time: per input shape the whole forward is compiled into a fixed launch sequence
 (optionally a CUDA graph), with skip connections and `Concat` resolved to buffer aliasing.
-Training-side members (loss, criterion, augment/TTA, profiling, Ensemble) are out of scope.
+Test-time augmentation (`augment=True`, reference `DetectionModel._predict_augment`) runs the plans of its three input
+shapes with two CUDA kernels around them (csrc/tta.cu).  Training-side members (loss, criterion, profiling, Ensemble)
+are out of scope.
 """
 from __future__ import annotations
 
@@ -15,6 +17,7 @@ import math
 import re
 from copy import deepcopy
 from pathlib import Path
+from typing import NamedTuple
 
 import torch
 import torch.nn as nn
@@ -134,6 +137,51 @@ def initialize_weights(model: nn.Module):
             m.inplace = True
 
 
+#: scales and flips of DetectionModel._predict_augment (flip 3 = left-right); the reference hard-codes both
+TTA_SCALES = (1, 0.83, 0.67)
+TTA_FLIPS = (None, 3, None)
+
+
+class TtaPass(NamedTuple):
+    """Geometry of one pass of _predict_augment on an (h, w) input."""
+
+    scale: float
+    flip: int | None
+    h: int            # resized content: (int(h * scale), int(w * scale)) as scale_img computes it
+    w: int
+    H: int            # canvas after scale_img's pad to a multiple of the largest stride
+    W: int
+    A: int            # anchors the model predicts on the canvas
+    a0: int           # anchors [a0, a0 + n) survive _clip_augmented
+    n: int
+
+
+def tta_geometry(h: int, w: int, strides=(8, 16, 32)) -> list[TtaPass]:
+    """The three passes of _predict_augment for an (h, w) input (a multiple of max(strides)): scale_img's content and
+    canvas sizes (utils/torch_utils.py, Python double arithmetic as there) and the anchor ranges _clip_augmented keeps
+    (the largest-stride level of the first pass and the smallest-stride level of the last pass are dropped)."""
+    strides = [int(s) for s in strides]
+    gs, nl = max(strides), len(strides)
+    g = sum(4 ** x for x in range(nl))         # _clip_augmented: anchors per unit of the smallest level
+    e = 1                                      # levels dropped at each end
+    out = []
+    for k, (si, fi) in enumerate(zip(TTA_SCALES, TTA_FLIPS)):
+        if si == 1.0:                          # scale_img returns the image unchanged
+            ch, cw, H, W = h, w, h, w
+        else:
+            ch, cw = int(h * si), int(w * si)
+            H, W = (math.ceil(x * si / gs) * gs for x in (h, w))
+        A = sum((H // s) * (W // s) for s in strides)
+        a0, n = 0, A
+        if k == 0:
+            n = A - (A // g) * sum(4 ** x for x in range(e))
+        elif k == len(TTA_SCALES) - 1:
+            a0 = (A // g) * sum(4 ** (nl - 1 - x) for x in range(e))
+            n = A - a0
+        out.append(TtaPass(si, fi, ch, cw, H, W, A, a0, n))
+    return out
+
+
 def fused_up_guard(layers):
     """Indices of layers whose output feeds an nn.Upsample (those producers need the dual-destination conv)."""
     out = set()
@@ -161,8 +209,13 @@ class BaseModel(YLModule):
         return self.predict(x, *args, **kwargs)
 
     def predict(self, x, profile=False, visualize=False, augment=False, embed=None):
-        if augment or visualize or embed or profile:
-            raise NotImplementedError("augment / visualize / embed / profile are not part of the inference hot path")
+        """Module-level forward: (y (B, 4+nc, A), [raw (B, no, H, W)]) like the reference; with `augment=True` the
+        merged test-time-augmentation prediction and None, like `_predict_augment`."""
+        if visualize or embed or profile:
+            raise NotImplementedError("visualize / embed / profile are not part of the inference hot path")
+        if augment and self._augment_supported():
+            y, _ = self.infer(x, augment=True)
+            return (y.clone() if self.clone_outputs else y), None
         out = self.infer(x, want_raw=True)   # the module-level API returns the raw head maps like the reference
         if self.clone_outputs:
             y, raws = out
@@ -362,8 +415,11 @@ class BaseModel(YLModule):
         return entry
 
     @torch.no_grad()
-    def infer(self, x: torch.Tensor, want_raw: bool = False, slot: int = 0):
+    def infer(self, x: torch.Tensor, want_raw: bool = False, slot: int = 0, augment: bool = False):
         """Engine entry: NCHW float image batch on CUDA -> (y (B, 4+nc, A) fp32, [raw (B, no, H, W) views]).
+
+        `augment=True`: test-time augmentation (reference `_predict_augment`) -> (merged (B, 4+nc, A_tta), []), boxes in
+        the pixels of `x`; `merged` aliases a buffer of this (shape, device, slot) that the next such call overwrites.
 
         `slot` selects one of several independent plans (own activation buffers and CUDA graph) for the same
         shape, so a caller can keep two batches in flight on two streams: the launch-latency-bound small layers
@@ -384,9 +440,64 @@ class BaseModel(YLModule):
         s = int(self.stride.max()) if hasattr(self, "stride") else 32
         if x.shape[2] % s or x.shape[3] % s:
             raise ValueError(f"image size {tuple(x.shape[2:])} must be a multiple of the model stride {s}")
+        if augment and self._augment_supported():
+            return self._infer_tta(x, dev, slot)["merged"], []
         plan, static_in, y, raws = self._get_plan(x.shape, dev, want_raw, slot)
         self._run_plan(plan, static_in, x, dev)
         return y, raws
+
+    # ------------------------------------------------------------------ test-time augmentation
+    def _augment_supported(self) -> bool:
+        """Only a detection model has the TTA path; anything else predicts single-scale with the reference's warning."""
+        if isinstance(self.model[-1], Detect) and not getattr(self, "end2end", False):
+            return True
+        LOGGER.warning("WARNING: Model does not support 'augment=True', reverting to single-scale prediction.")
+        return False
+
+    def _infer_tta(self, x, dev, slot):
+        """_predict_augment on the engine path: pass 0 is the plain plan of `x` (same ingest, uint8 / fp16 read natively),
+        yl_tta_scale_img writes the flipped / rescaled inputs of passes 1 and 2 straight into their plans' static inputs,
+        the two plans replay, and yl_tta_merge builds the merged prediction in a buffer of the returned TTA state (keyed
+        and bounded like the plans).  Asynchronous: nothing here waits for the device."""
+        from .. import _C, _ops
+
+        B, C, H, W = x.shape
+        geo = tta_geometry(H, W, self.model[-1].stride.tolist())
+        plans, shapes = [], []
+        for k, p in enumerate(geo):
+            shape = (B, C, p.H, p.W)
+            # the three outputs must coexist until the merge: a canvas equal to an earlier pass's shape (small inputs,
+            # where the rescaled canvas pads back to the same size) gets a plan slot of its own; callers use slots >= 0
+            plans.append(self._get_plan(shape, dev, False, slot if shape not in shapes else -(3 * int(slot) + k)))
+            shapes.append(shape)
+        for (_, _, y, _), p in zip(plans, geo):
+            assert y.shape[2] == p.A, (tuple(y.shape), p)
+        st = self._tta_state(x.shape, dev, slot, plans[0][2].shape[1], sum(p.n for p in geo))
+        plan0, in0, _, _ = plans[0]
+        self._run_plan(plan0, in0, x, dev)
+        xs = x if x.dtype in _C.INGEST_DTYPES else x.float()
+        xs = xs if xs.is_contiguous() else xs.contiguous()
+        with torch.cuda.device(dev):
+            _ops.tta_scale_img(xs, [(plans[k][1], (geo[k].h, geo[k].w), geo[k].flip) for k in (1, 2)])
+            plans[1][0].run()
+            plans[2][0].run()
+            _ops.tta_merge([(plans[k][2], p.a0, p.n, p.scale, p.flip) for k, p in enumerate(geo)], W, st["merged"])
+        return st
+
+    def _tta_state(self, shape, dev, slot, rows, anchors):
+        """Output buffers of test-time augmentation for one (input shape, device, slot): the merged prediction and the
+        NMS outputs per argument set.  LRU-bounded by `max_plans`, like the plans."""
+        states = self.__dict__.setdefault("_yl_tta", {})
+        key = (tuple(shape), dev.index, int(slot))
+        st = states.get(key)
+        if st is not None:
+            states[key] = states.pop(key)
+            return st
+        if len(states) >= max(int(self.max_plans), 1):
+            torch.cuda.synchronize(dev)          # the evicted buffers may still be in use on some stream
+            states.pop(next(iter(states)))
+        st = states[key] = {"merged": torch.empty((shape[0], rows, anchors), dtype=torch.float32, device=dev), "nms": {}}
+        return st
 
     @staticmethod
     def _run_plan(plan, static_in, x, dev):
@@ -411,11 +522,14 @@ class BaseModel(YLModule):
 
     @torch.no_grad()
     def infer_nms(self, x: torch.Tensor, conf=0.25, iou=0.45, classes=None, agnostic=False, multi_label=False,
-                  max_det=300, max_nms=30000, max_wh=7680.0, slot: int = 0):
+                  max_det=300, max_nms=30000, max_wh=7680.0, slot: int = 0, augment: bool = False):
         """Engine entry for a whole step: NCHW float batch on CUDA -> (dets (B, max_det, 6), counts (B,) int32), the
         padded output of `ops.nms_padded(self.infer(x)[0], ...)`, with the NMS kernels recorded in the same plan /
         CUDA graph as the model (ingest + one graph launch per step).  The returned tensors alias plan buffers and
-        are overwritten by the next call with the same shape, arguments and slot."""
+        are overwritten by the next call with the same shape, arguments and slot.
+
+        `augment=True`: the same NMS on the merged test-time-augmentation prediction of `infer(x, augment=True)`, into
+        buffers of its TTA state (same aliasing rule)."""
         if not isinstance(x, torch.Tensor) or x.dim() != 4 or not x.is_cuda:
             raise RuntimeError("infer_nms expects a (B, C, H, W) CUDA tensor (yololite has no CPU fallback)")
         dev = x.device
@@ -426,6 +540,22 @@ class BaseModel(YLModule):
             classes = [classes] if isinstance(classes, int) else list(classes)      # `classes=0` is legal in the reference
         nms = (float(conf), float(iou), None if classes is None else tuple(int(c) for c in classes), bool(agnostic),
                bool(multi_label), int(max_det), int(max_nms), float(max_wh))
+        if augment and self._augment_supported():
+            from .. import _ops
+
+            st = self._infer_tta(x, dev, slot)
+            out = st["nms"].pop(nms, None)
+            if out is None:
+                if len(st["nms"]) >= max(int(self.max_plans), 1):
+                    torch.cuda.synchronize(dev)
+                    st["nms"].pop(next(iter(st["nms"])))
+                cls_t = None if nms[2] is None else torch.tensor(nms[2], dtype=torch.int32, device=dev)
+                out = (torch.empty((x.shape[0], nms[5], 6), dtype=torch.float32, device=dev),
+                       torch.empty((x.shape[0],), dtype=torch.int32, device=dev), cls_t)
+            st["nms"][nms] = out                 # most recently used last
+            with torch.cuda.device(dev):
+                return _ops.nms_batched(st["merged"], conf, iou, out[2], agnostic, multi_label, max_det, max_nms, max_wh,
+                                        out=out[0], counts=out[1])
         plan, static_in, _, post = self._get_plan(x.shape, dev, False, slot, nms)
         self._run_plan(plan, static_in, x, dev)
         return post
