@@ -366,6 +366,23 @@ typedef struct yl_tta_pass {
  * `p[:, :4] /= scale`) and, for a flipped pass, row 0 replaced by img_w - x.  Bit-identical to those torch ops on CUDA. */
 int yl_tta_merge(const yl_tta_pass* passes, int B, int nc, int img_w, float* y, void* stream);
 
+/* ---- feature embeddings (BaseModel._predict_once with `embed`, nn/tasks.py) ------------------------------------ */
+/* One tapped layer output: an NHWC bf16 channel slice (c, coff and cstride multiples of 8, data 16-byte aligned) whose
+ * per-channel spatial mean fills output columns [col, col + c). */
+typedef struct yl_embed_tap {
+    yl_tensor x;
+    int32_t col;
+    int32_t _pad;
+} yl_embed_tap;
+/* adaptive_avg_pool2d(x, (1, 1)).squeeze(-1).squeeze(-1) of every tap, side by side in out (B, D) fp32, in ONE launch:
+ * each element is the fp32 sum of the tap's h*w bf16 values times 1/(h*w).  taps: n_taps (<= 32) descriptors in HOST
+ * memory, each with n == B.  Deterministic (no floating-point atomics; the pixel split is a function of h*w and c only).
+ * workspace: NULL -> only writes the bytes it needs to *workspace_bytes (0 is possible) and returns.  Otherwise
+ * *workspace_bytes is its capacity; it must be zeroed once before its first use, and every completed launch leaves it
+ * zeroed again.  One workspace serves one launch at a time. */
+int yl_embed_pool(const yl_embed_tap* taps, int n_taps, int B, int D, float* out, void* workspace, size_t* workspace_bytes,
+                  void* stream);
+
 #ifdef __cplusplus
 }
 #endif

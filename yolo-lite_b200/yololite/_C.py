@@ -125,6 +125,12 @@ class TtaPass(C.Structure):
                 ("scale", C.c_float), ("_pad", C.c_int32)]
 
 
+class EmbedTap(C.Structure):
+    """Mirror of `yl_embed_tap` (48 bytes)."""
+
+    _fields_ = [("x", Tensor), ("col", C.c_int32), ("_pad", C.c_int32)]
+
+
 _PROTOTYPES = {
     "yl_version": (C.c_int, []),
     "yl_last_error_string": (C.c_char_p, []),
@@ -189,6 +195,8 @@ _PROTOTYPES = {
     "yl_tta_scale_img": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(TtaCanvas),
                                    C.c_void_p]),
     "yl_tta_merge": (C.c_int, [C.POINTER(TtaPass), C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "yl_embed_pool": (C.c_int, [C.POINTER(EmbedTap), C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                C.POINTER(C.c_size_t), C.c_void_p]),
 }
 
 EXPORTS = tuple(_PROTOTYPES)

@@ -295,3 +295,35 @@ def tta_merge(passes, img_w: int, out: torch.Tensor) -> torch.Tensor:
                              for p, a0, n, s, flip in passes])
     _C.check(_C.load().yl_tta_merge(arr, B, C4 - 4, int(img_w), out.data_ptr(), _C.stream_ptr()), "yl_tta_merge")
     return out
+
+
+def embed_pool_taps(views):
+    """yl_embed_tap array of NHWC bf16 channel slices whose pooled means fill consecutive output columns, and the total
+    width D."""
+    arr = (_C.EmbedTap * len(views))()
+    col = 0
+    for k, v in enumerate(views):
+        arr[k] = _C.EmbedTap(v.ct(), col, 0)
+        col += v.c
+    return arr, col
+
+
+def embed_pool_workspace(taps, B: int, D: int, device) -> torch.Tensor:
+    """Zeroed workspace of yl_embed_pool for these taps (at least 16 bytes)."""
+    need = C.c_size_t(0)
+    _C.check(_C.load().yl_embed_pool(taps, len(taps), B, D, None, None, C.byref(need), None), "yl_embed_pool")
+    return torch.zeros(max(int(need.value), 16), dtype=torch.uint8, device=device)
+
+
+def embed_pool(views, out: torch.Tensor, workspace: torch.Tensor | None = None) -> torch.Tensor:
+    """Per-channel spatial mean of every view (adaptive_avg_pool2d to 1x1), side by side in out (B, sum of c) fp32, in one
+    launch (yl_embed_pool).  `workspace`: from embed_pool_workspace for the same views (allocated here when None)."""
+    taps, D = embed_pool_taps(views)
+    B = views[0].n
+    assert out.is_cuda and out.dtype == torch.float32 and out.is_contiguous() and tuple(out.shape) == (B, D)
+    if workspace is None:
+        workspace = embed_pool_workspace(taps, B, D, out.device)
+    cap = C.c_size_t(workspace.numel())
+    _C.check(_C.load().yl_embed_pool(taps, len(taps), B, D, out.data_ptr(), workspace.data_ptr(), C.byref(cap),
+                                     _C.stream_ptr()), "yl_embed_pool")
+    return out

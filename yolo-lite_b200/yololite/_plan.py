@@ -74,6 +74,7 @@ class Builder:
         # filter in its conv epilogues (set by BaseModel._get_plan); the head then fills `cand_ws`
         self.nms_fuse_conf: float | None = None
         self.cand_ws: torch.Tensor | None = None
+        self.layer: int | None = None      # model layer being emitted (recorded in `meta`; set by BaseModel._emit)
         # conv chains (csrc/conv_chain.cu): runs of small-map convs as ONE launch, one 4-CTA cluster per image.  Opt-in
         # (YL_CHAIN=1): parity-exact, but measured 3-5 % slower than the per-layer launches at every batch size — those
         # layers are bound by L2 -> SM operand traffic and the per-MMA A-operand read, not by launch overhead
@@ -139,7 +140,8 @@ class Builder:
         self.lanes.append(self._cur_lane)
         self.deps.append(self._track(idx, reads, writes))
         # algorithmic work of the launch (each operand touched once): the roofline numerators of DESIGN.md
-        self.meta.append({"kind": kind or fn.__name__, "bytes": int(bytes_), "flops": int(flops), "desc": desc})
+        self.meta.append({"kind": kind or fn.__name__, "bytes": int(bytes_), "flops": int(flops), "desc": desc,
+                          "layer": self.layer})
 
     # ------------------------------------------------------------------ ops
     def input_nchw(self, x_nchw_static: torch.Tensor) -> NchwInput:
@@ -418,6 +420,21 @@ class Builder:
                    counts.data_ptr(), keep=(ws, out, counts, cls_t, pred), kind="nms", bytes_=B * C4 * A * 4,
                    desc=f"conf {conf} iou {iou} max_det {max_det}", reads=(pred,), writes=(out, counts, ws))
         return out, counts
+
+    def embed_pool(self, views: list[View]) -> torch.Tensor:
+        """Per-channel spatial means of the tapped layer outputs `views`, side by side in a plan-owned (B, D) fp32 output
+        (yl_embed_pool, one launch ordered after every producer of the taps)."""
+        B = views[0].n
+        taps, D = _ops.embed_pool_taps(views)
+        out = torch.empty((B, D), dtype=torch.float32, device=self.device)
+        ws = _ops.embed_pool_workspace(taps, B, D, self.device)
+        self.buffers += [out, ws]
+        cap = C.c_size_t(ws.numel())
+        self._push(self.lib.yl_embed_pool, taps, len(views), B, D, out.data_ptr(), ws.data_ptr(), C.byref(cap),
+                   keep=(taps, cap, ws, out), kind="embed_pool",
+                   bytes_=sum(v.n * v.h * v.w * v.c * 2 for v in views) + B * D * 4,
+                   desc=f"{len(views)} taps -> ({B}, {D}) f32", reads=tuple(views), writes=(out, ws))
+        return out
 
     def to_nchw(self, x: View) -> torch.Tensor:
         x = self.mat(x)

@@ -70,6 +70,13 @@ class YOLOLite(nn.Module):
             self.predictor = predictor
         return self.predictor(source=source, stream=stream)
 
+    def embed(self, source=None, stream: bool = False, **kwargs):
+        """Image feature vectors (reference Model.embed): `predict` with `embed` defaulting to the last layer before the
+        head (22 for YOLO11; 256 values per image for yolo11n).  Yields / returns one 1-D fp32 tensor per image."""
+        if not kwargs.get("embed"):
+            kwargs["embed"] = [len(self.model.model) - 2]
+        return self.predict(source, stream, **kwargs)
+
     def val(self, dataloader=None, **kwargs):
         """Validate on labelled batches (reference engine/model.py:101-107).  `dataloader`: iterable of batch dicts in
         the reference's collate layout; or `data=<dataset yaml | image dir>`: the split is loaded with the minimal rect

@@ -8,6 +8,8 @@ per batch, yielding `Results`.  The three stages keep the reference's names and 
   * a HOST tensor batch is ingested in chunks: chunk k+1's host->device copy runs on a copy stream while the
     model + NMS of chunk k run on the compute stream, so the PCIe transfer (the e2e bound for fp32 images:
     4.9 MB per 640x640 image) overlaps the whole GPU pipeline instead of preceding it;
+  * `embed=[layer indices]` yields one feature vector (1-D fp32 tensor) per image instead of `Results`, as the
+    reference's stream loop does; the model runs only up to the last tapped layer (`BaseModel.infer_embed`);
   * saving / plotting / video writing (predictor.py:248-323) are I/O features outside the hot path.
 """
 from __future__ import annotations
@@ -21,6 +23,7 @@ from .. import _C
 from ..cfg import DEFAULT_CFG, get_cfg
 from ..data import LetterBox, load_inference_source
 from ..nn.autobackend import AutoBackend
+from ..nn.tasks import embed_indices
 from ..utils import LOGGER, ops
 from ..utils.torch_utils import select_device, smart_inference_mode
 from .results import BatchDetections, Results
@@ -44,6 +47,9 @@ class DetectionPredictor:
         self.args = get_cfg(cfg, overrides)
         if self.args.conf is None:
             self.args.conf = 0.25
+        if self.args.embed and self.args.augment:
+            # the reference would yield the merged TTA prediction and then None in place of feature vectors
+            raise ValueError("embed and augment=True cannot be combined: embeddings come from a single-scale pass")
         if self.args.save or self.args.save_txt or self.args.save_crop or self.args.show:
             if self.args.verbose:
                 LOGGER.info("save/show requested: result files and plots are outside yololite's scope; ignored")
@@ -118,14 +124,17 @@ class DetectionPredictor:
 
     def _pipelined(self, im_host, n_chunks):
         """preprocess + inference + NMS of a host fp32 batch, chunk-pipelined.  Returns (device batch, dets,
-        counts); the detections of chunk k land in rows [k*cb, (k+1)*cb) of the batch-level outputs."""
+        counts); the detections of chunk k land in rows [k*cb, (k+1)*cb) of the batch-level outputs.  With `embed`
+        set: (device batch, (B, D) embeddings, None), chunk k's feature vectors in rows [k*cb, (k+1)*cb)."""
         a = self.args
         dev = self.device
         B = im_host.shape[0]
         cb = B // n_chunks
+        model = self.model.model
+        emb = embed_indices(a.embed, len(model.model)) if a.embed else None
         # fp16 / uint8 batches stay narrow all the way into the model's ingest kernel (2x / 4x fewer PCIe and HBM bytes);
         # uint8 means image bytes and is scaled by 1/255 there (reference predictor.py:83-84: `.float()`, `/= 255`)
-        key = (tuple(im_host.shape), a.max_det, str(im_host.dtype))
+        key = (tuple(im_host.shape), a.max_det, str(im_host.dtype), emb)
         # the staging state lives on the backend: YOLOLite.predict builds a fresh predictor per call, but the pinned
         # upload pipeline (two device staging batches, streams, events) must survive across calls.  The side streams
         # are shared by every state; buffers are kept per (shape, max_det, dtype) in a small LRU so that alternating
@@ -149,9 +158,13 @@ class DetectionPredictor:
                 states.pop(next(iter(states)))
             st = {"key": key, "bufs": [torch.empty(im_host.shape, dtype=im_host.dtype, device=dev) for _ in range(2)],
                   "free": [None, None], "turn": 0,
-                  "dets": torch.empty((B, a.max_det, 6), dtype=torch.float32, device=dev),
-                  "counts": torch.empty((B,), dtype=torch.int32, device=dev),
                   "events": [torch.cuda.Event() for _ in range(n_chunks)]}
+            if emb is None:
+                st["dets"] = torch.empty((B, a.max_det, 6), dtype=torch.float32, device=dev)
+                st["counts"] = torch.empty((B,), dtype=torch.int32, device=dev)
+            else:
+                D = sum(model._out_channels(list(model.model), k, {}) for k in emb)
+                st["emb"] = torch.empty((B, D), dtype=torch.float32, device=dev)
             states[key] = st
         st["copy"], st["lanes"], st["post"] = pipe["copy"], pipe["lanes"], pipe["post"]
         self.model.__dict__["_yl_pipe_state"] = st       # the state the most recent call used
@@ -175,7 +188,6 @@ class DetectionPredictor:
             for k in range(n_chunks):
                 buf[k * cb:(k + 1) * cb].copy_(im_host[k * cb:(k + 1) * cb], non_blocking=True)
                 st["events"][k].record(st["copy"])
-        model = self.model.model
         fly = max(1, min(int(self.in_flight), 2))
         lanes = st["lanes"][:fly]
         lane0 = pipe.get("next_lane", 0)         # chunks (and single-chunk calls) keep alternating lanes across calls
@@ -185,6 +197,12 @@ class DetectionPredictor:
             ln = lanes[li]
             with torch.cuda.stream(ln):
                 ln.wait_event(st["events"][k])
+                if emb is not None:
+                    e = model.infer_embed(buf[k * cb:(k + 1) * cb], emb, slot=li)
+                    if pipe["snap"] is not None:
+                        ln.wait_event(pipe["snap"])
+                    st["emb"][k * cb:(k + 1) * cb].copy_(e, non_blocking=True)
+                    continue
                 # model + NMS of the chunk are one CUDA-graph launch; its plan-owned outputs are gathered into the
                 # batch-level buffers (115 KB per 16 images)
                 d, c = model.infer_nms(buf[k * cb:(k + 1) * cb], a.conf, a.iou, a.classes, a.agnostic_nms, False,
@@ -198,7 +216,22 @@ class DetectionPredictor:
             post.wait_stream(ln)
         st["free"][j] = torch.cuda.Event()
         st["free"][j].record(post)
+        if emb is not None:
+            return buf, st["emb"], None, post
         return buf, st["dets"], st["counts"], post
+
+    def _embed_rows(self, emb, stream=None):
+        """Per-image rows of one clone of the (B, D) embeddings, taken on the current stream (after `stream`, the
+        pipeline's post stream, when given)."""
+        cur = torch.cuda.current_stream(self.device)
+        if stream is not None:
+            cur.wait_stream(stream)
+        rows = torch.unbind(emb.clone(), 0)
+        if stream is not None:
+            pipe = self.model.__dict__["_yl_pipe"]
+            pipe["snap"] = torch.cuda.Event()    # the next pipelined call may overwrite the batch-level buffer after this
+            pipe["snap"].record(cur)
+        return rows
 
     def postprocess(self, preds, img, orig_imgs, nms_out=None, stream=None):
         """`stream`: run the rescale + snapshot there (the asynchronous host-tensor pipeline) instead of on the
@@ -278,6 +311,9 @@ class DetectionPredictor:
                     # host tensor batch: copy / model / NMS run chunk-pipelined (preprocess+inference timed together)
                     with profilers[1]:
                         im, dets, counts, post = self._pipelined(im0s, n_chunks)
+                    if self.args.embed:
+                        yield from self._embed_rows(dets, post)
+                        continue
                     profilers[0].dt = 0.0
                     with profilers[2]:
                         self.results = self.postprocess(None, im, im0s, nms_out=(dets, counts), stream=post)
@@ -289,8 +325,13 @@ class DetectionPredictor:
                             cur.wait_stream(side)
                     with profilers[0]:
                         im = self.preprocess(im0s)
+                    a = self.args
+                    if a.embed:                 # the reference's stream loop yields the feature vectors, no postprocess
+                        with profilers[1]:
+                            rows = self._embed_rows(self.model.model.infer_embed(im, a.embed))
+                        yield from rows
+                        continue
                     with profilers[1]:
-                        a = self.args
                         nms_out = self.model.model.infer_nms(im, a.conf, a.iou, a.classes, a.agnostic_nms, False, a.max_det,
                                                              augment=a.augment)
                     with profilers[2]:

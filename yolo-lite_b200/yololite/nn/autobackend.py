@@ -45,9 +45,14 @@ class AutoBackend(nn.Module):
         self.batch = batch
 
     def forward(self, im, augment=False, visualize=False, embed=None):
-        """[y, raw maps]; with `augment=True` [merged test-time-augmentation prediction, None]."""
-        if visualize or embed:
-            raise NotImplementedError("visualize / embed are not part of the inference hot path")
+        """[y, raw maps]; with `augment=True` [merged test-time-augmentation prediction, None].  With `embed=[layer
+        indices]` and no `augment` (which wins, as in the reference) the per-image feature vectors of
+        `model.infer_embed`: a list of B 1-D tensors, or the tensor itself when B == 1."""
+        if visualize:
+            raise NotImplementedError("visualize is not part of the inference hot path")
+        if embed and not augment:
+            y = torch.unbind(self.model.infer_embed(im, embed), 0)
+            return y[0] if len(y) == 1 else list(y)
         y, raws = self.model.infer(im, augment=augment)
         return [y, None] if augment else [y, raws]
 

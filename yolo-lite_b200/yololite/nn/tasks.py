@@ -7,8 +7,9 @@ Public surface follows reference yololite/nn/tasks.py: `DetectionModel(cfg, ch, 
 exists only at plan-build time: per input shape the whole forward is compiled into a fixed launch sequence
 (optionally a CUDA graph), with skip connections and `Concat` resolved to buffer aliasing.
 Test-time augmentation (`augment=True`, reference `DetectionModel._predict_augment`) runs the plans of its three input
-shapes with two CUDA kernels around them (csrc/tta.cu).  Training-side members (loss, criterion, profiling, Ensemble)
-are out of scope.
+shapes with two CUDA kernels around them (csrc/tta.cu).  Feature embeddings (`embed=[...]`) run a plan truncated after
+the last tapped layer that ends in one pooling kernel (csrc/embed.cu).  Training-side members (loss, criterion,
+profiling, Ensemble) are out of scope.
 """
 from __future__ import annotations
 
@@ -182,6 +183,26 @@ def tta_geometry(h: int, w: int, strides=(8, 16, 32)) -> list[TtaPass]:
     return out
 
 
+def embed_indices(embed, n_layers: int) -> tuple[int, ...]:
+    """The layer indices of `embed` as the plan key: sorted and de-duplicated (the reference's `m.i in embed` test pools
+    in layer order and counts a repeated index once).  Unlike the reference, an index outside [0, n_layers - 2] raises
+    ValueError: the last layer (Detect) returns a list the reference cannot pool, and the reference silently ignores a
+    negative index and then returns detections."""
+    if isinstance(embed, (str, bytes)) or not hasattr(embed, "__iter__"):
+        raise TypeError(f"embed must be a list of layer indices, got {embed!r}")
+    idx = set()
+    for i in embed:
+        if isinstance(i, bool) or not hasattr(i, "__index__"):
+            raise TypeError(f"embed index {i!r} is not an int")
+        i = i.__index__()
+        if not 0 <= i <= n_layers - 2:
+            raise ValueError(f"embed index {i} is outside [0, {n_layers - 2}] (layers 0..{n_layers - 2} precede the head)")
+        idx.add(i)
+    if not idx:
+        raise ValueError("embed needs at least one layer index")
+    return tuple(sorted(idx))
+
+
 def fused_up_guard(layers):
     """Indices of layers whose output feeds an nn.Upsample (those producers need the dual-destination conv)."""
     out = set()
@@ -210,12 +231,17 @@ class BaseModel(YLModule):
 
     def predict(self, x, profile=False, visualize=False, augment=False, embed=None):
         """Module-level forward: (y (B, 4+nc, A), [raw (B, no, H, W)]) like the reference; with `augment=True` the
-        merged test-time-augmentation prediction and None, like `_predict_augment`."""
-        if visualize or embed or profile:
-            raise NotImplementedError("visualize / embed / profile are not part of the inference hot path")
+        merged test-time-augmentation prediction and None, like `_predict_augment`.  With `embed=[layer indices]` (and
+        no `augment`, which wins as in the reference) the tuple of B per-image feature vectors of `_predict_once`: the
+        per-channel spatial means of the tapped layers' outputs, concatenated in layer order (see `infer_embed`)."""
+        if visualize or profile:
+            raise NotImplementedError("visualize / profile are not part of the inference hot path")
         if augment and self._augment_supported():
             y, _ = self.infer(x, augment=True)
             return (y.clone() if self.clone_outputs else y), None
+        if embed:
+            e = self.infer_embed(x, embed)
+            return torch.unbind(e.clone() if self.clone_outputs else e, 0)
         out = self.infer(x, want_raw=True)   # the module-level API returns the raw head maps like the reference
         if self.clone_outputs:
             y, raws = out
@@ -246,9 +272,13 @@ class BaseModel(YLModule):
             sc.append(s)
         return sc
 
-    def _emit(self, g, x, out=None):
+    def _emit(self, g, x, out=None, embed=None):
         """Record the whole forward. Concat layers whose inputs each feed exactly one Concat become aliasing:
-        the producers are handed a slice of the concat buffer as their destination."""
+        the producers are handed a slice of the concat buffer as their destination.
+
+        `embed`: sorted layer indices (embed_indices).  Only layers 0..max(embed) are recorded, and the return value is
+        the list of the tapped layers' output Views (a buffer, a concat slice, a Concat's whole buffer or a fused
+        upsample's replicated copy)."""
         from .._ops import View
 
         layers = list(self.model)
@@ -301,14 +331,20 @@ class BaseModel(YLModule):
         for u, m in enumerate(layers):
             if isinstance(m, nn.Upsample) and m.mode == "nearest" and float(m.scale_factor) == 2.0:
                 j = srcs[u][0]
+                if embed is not None and u > embed[-1]:
+                    continue             # the upsample is never emitted: its producer writes only its plain output
                 if j >= 0 and isinstance(layers[j], (Conv, C2f, C3, SPPF, C2PSA)) and j not in fused_up:
                     fused_up[j] = u
         done_up = {}
 
         # layers 0 + 1 as one launch (image ingest + two stride-2 3x3 convs) when layer 0 feeds only layer 1
-        fuse_stem = self._stem_fusable(g, x, layers, srcs, n_uses)
+        # (layer 0's output never leaves shared memory there, so a tap on it takes the unfused stem)
+        fuse_stem = not (embed is not None and 0 in embed) and self._stem_fusable(g, x, layers, srcs, n_uses)
         cur = x
         for i, m in enumerate(layers):
+            if embed is not None and i > embed[-1]:
+                return [ys[k] for k in embed]
+            g.layer = i
             if fuse_stem and i == 0:
                 continue
             if fuse_stem and i == 1:
@@ -383,11 +419,13 @@ class BaseModel(YLModule):
         memo[k] = c
         return c
 
-    def _get_plan(self, shape, dev, want_raw=False, slot=0, nms=None):
+    def _get_plan(self, shape, dev, want_raw=False, slot=0, nms=None, embed=None):
         """`nms`: None or the hashable argument tuple of Builder.nms: the plan then ends with the batched NMS and its
-        entry carries (dets, counts) instead of the raw head maps."""
+        entry carries (dets, counts) instead of the raw head maps.  `embed`: None or the index tuple of embed_indices:
+        the plan stops after layer max(embed) and ends with the pooling launch; its entry carries the (B, D) fp32
+        embeddings in place of `y` and no raw maps."""
         plans = self.__dict__.setdefault("_yl_plans", {})
-        key = (tuple(shape), dev.index, bool(self.use_cuda_graph), bool(want_raw), int(slot), nms)
+        key = (tuple(shape), dev.index, bool(self.use_cuda_graph), bool(want_raw), int(slot), nms, embed)
         entry = plans.get(key)
         if entry is not None:
             plans[key] = plans.pop(key)                     # most recently used last (dicts keep insertion order)
@@ -404,7 +442,10 @@ class BaseModel(YLModule):
                     g.nms_fuse_conf = float(nms[0])   # single-label, no class filter: the head may filter in its epilogue
                 static_in = torch.zeros(tuple(shape), dtype=torch.float32, device=dev)
                 xin = g.input_nchw(static_in)
-                y, raws = self._emit(g, xin)
+                if embed is not None:
+                    y, raws = g.embed_pool(self._emit(g, xin, embed=embed)), []
+                else:
+                    y, raws = self._emit(g, xin)
                 post = g.nms(y, *nms) if nms is not None else None
                 plan = g.finish()
                 if self.use_cuda_graph:
@@ -428,6 +469,15 @@ class BaseModel(YLModule):
         The raw head maps are only needed by callers of the module-level API (`forward`); the engine path
         (`want_raw=False`) gets an empty list and the plan never writes them.  The returned tensors alias the
         plan's static buffers and are overwritten by the next call with the same shape."""
+        dev = self._engine_device(x)
+        if augment and self._augment_supported():
+            return self._infer_tta(x, dev, slot)["merged"], []
+        plan, static_in, y, raws = self._get_plan(x.shape, dev, want_raw, slot)
+        self._run_plan(plan, static_in, x, dev)
+        return y, raws
+
+    def _engine_device(self, x) -> torch.device:
+        """The device of an engine-entry batch, after the checks every entry makes."""
         if not isinstance(x, torch.Tensor) or x.dim() != 4:
             raise TypeError("expected a (B, C, H, W) tensor")
         if not x.is_cuda:
@@ -440,11 +490,21 @@ class BaseModel(YLModule):
         s = int(self.stride.max()) if hasattr(self, "stride") else 32
         if x.shape[2] % s or x.shape[3] % s:
             raise ValueError(f"image size {tuple(x.shape[2:])} must be a multiple of the model stride {s}")
-        if augment and self._augment_supported():
-            return self._infer_tta(x, dev, slot)["merged"], []
-        plan, static_in, y, raws = self._get_plan(x.shape, dev, want_raw, slot)
+        return dev
+
+    @torch.no_grad()
+    def infer_embed(self, x: torch.Tensor, embed, slot: int = 0) -> torch.Tensor:
+        """Engine entry for feature embeddings: NCHW image batch on CUDA (fp32, fp16 or uint8 bytes, read like `infer`)
+        -> (B, D) fp32, row b the embedding of image b: for every layer index of `embed` in layer order (repeats count
+        once) the per-channel spatial mean of that layer's output, D the sum of their channel counts.  That is the
+        reference's `_predict_once(x, embed=...)`: the plan records layers 0..max(embed) only, then one yl_embed_pool
+        launch.  Indices must lie in [0, len(model) - 2] (ValueError otherwise, see embed_indices).  The result
+        aliases a buffer of this plan (shape, device, slot, indices) that the next such call overwrites."""
+        dev = self._engine_device(x)
+        idx = embed_indices(embed, len(self.model))
+        plan, static_in, out, _ = self._get_plan(x.shape, dev, False, slot, embed=idx)
         self._run_plan(plan, static_in, x, dev)
-        return y, raws
+        return out
 
     # ------------------------------------------------------------------ test-time augmentation
     def _augment_supported(self) -> bool:
