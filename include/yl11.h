@@ -233,6 +233,12 @@ int yl_psa_attention(const yl_tensor* qkv, const yl_tensor* out, int heads, int 
  * row-major inside a level: y[:, :4] = (cx, cy, w, h) * stride, y[:, 4:] = sigmoid(cls). */
 int yl_detect_decode(const yl_tensor* levels, int nl, const float* strides_host, int reg_max, int nc, float* y,
                      void* stream);
+/* The same decode into a window of a wider prediction (the members of a model ensemble, Ensemble.forward nn/tasks.py,
+ * concatenate their predictions along the anchor axis): y is dense fp32 (B, 4+nc, y_anchors) and the A = sum h_i*w_i
+ * anchors land in columns [anchor_base, anchor_base + A); no other column is touched.  yl_detect_decode is this call
+ * with (A, 0). */
+int yl_detect_decode_into(const yl_tensor* levels, int nl, const float* strides_host, int reg_max, int nc, float* y,
+                          int y_anchors, int anchor_base, void* stream);
 
 /* Standalone DFL module (block.py:51-69): x dense fp32 (b, 4*reg_max, a) -> y (b, 4, a): softmax over the
  * reg_max bins of each side, expectation with weights 0..reg_max-1. */

@@ -1,6 +1,7 @@
 // Detect head decode: DFL softmax-expectation + anchor/dist2bbox + stride scale + class sigmoid in one pass
 // (head.py:95-126, block.py:51-69, tal.py:326-350).  Input: per-level raw maps NHWC f32 with 4*reg_max box
-// bins followed by nc class logits.  Output: (B, 4+nc, A) fp32, anchors level-major / row-major.
+// bins followed by nc class logits.  Output: (B, 4+nc, A) fp32, anchors level-major / row-major, or anchors
+// [anchor_base, anchor_base + A) of a wider (B, 4+nc, y_anchors) prediction (one member of a model ensemble).
 // A CTA takes 32 consecutive anchors of one image and level: the [32][no] tile is read with 16-B vectors
 // (contiguous in NHWC), transposed through padded shared memory, and every output channel row is written as
 // one 128-B coalesced segment.
@@ -36,14 +37,22 @@ __global__ void __launch_bounds__(256) detect_decode_kernel(const DecodeParams p
     const int no = nbox + p.nc;
     const int ld = no + 1;
 
-    // ---- load [cnt][no] (no % 4 == 0 is checked on the host)
-    const int v4 = no >> 2;
-    for (int i = threadIdx.x; i < cnt * v4; i += blockDim.x) {
-        const int px = i / v4, q = i - px * v4;
-        const float4 t = __ldg(reinterpret_cast<const float4*>(
-            p.x[lvl] + ((long long)b * HW + a0 + px) * p.cstride[lvl] + p.coff[lvl] + q * 4));
-        float* d = tile + px * ld + q * 4;
-        d[0] = t.x; d[1] = t.y; d[2] = t.z; d[3] = t.w;
+    // ---- load [cnt][no]: 16-B vectors when no, coff and cstride are multiples of 4 (checked on the host), else
+    // scalars (heads whose nc is not a multiple of 4)
+    const float* src = p.x[lvl] + ((long long)b * HW + a0) * p.cstride[lvl] + p.coff[lvl];
+    if ((no & 3) == 0) {
+        const int v4 = no >> 2;
+        for (int i = threadIdx.x; i < cnt * v4; i += blockDim.x) {
+            const int px = i / v4, q = i - px * v4;
+            const float4 t = __ldg(reinterpret_cast<const float4*>(src + (long long)px * p.cstride[lvl] + q * 4));
+            float* d = tile + px * ld + q * 4;
+            d[0] = t.x; d[1] = t.y; d[2] = t.z; d[3] = t.w;
+        }
+    } else {
+        for (int i = threadIdx.x; i < cnt * no; i += blockDim.x) {
+            const int px = i / no, q = i - px * no;
+            tile[px * ld + q] = __ldg(src + (long long)px * p.cstride[lvl] + q);
+        }
     }
     __syncthreads();
 
@@ -121,20 +130,19 @@ extern "C" int yl_dfl(const float* x, float* y, int b, int reg_max, int a, void*
     return YL_OK;
 }
 
-extern "C" int yl_detect_decode(const yl_tensor* levels, int nl, const float* strides_host, int reg_max, int nc,
-                                float* y, void* stream) {
+extern "C" int yl_detect_decode_into(const yl_tensor* levels, int nl, const float* strides_host, int reg_max, int nc,
+                                     float* y, int y_anchors, int anchor_base, void* stream) {
     YL_CHECK(levels && strides_host && y, YL_ERR_ARG, "null pointer");
     YL_CHECK(nl >= 1 && nl <= yl::kMaxLevels, YL_ERR_ARG, "1..%d levels supported", yl::kMaxLevels);
     YL_CHECK(reg_max >= 1 && nc >= 1, YL_ERR_ARG, "bad reg_max/nc");
     const int no = 4 * reg_max + nc;
-    YL_CHECK(no % 4 == 0, YL_ERR_UNSUPPORTED, "4*reg_max + nc must be a multiple of 4");
     yl::DecodeParams p;
     int tiles = 0, A = 0;
     for (int i = 0; i < nl; ++i) {
         const yl_tensor& t = levels[i];
         YL_CHECK(t.data && t.dtype == YL_F32, YL_ERR_ARG, "level %d must be f32", i);
-        YL_CHECK(t.c == no && t.coff % 4 == 0 && t.cstride % 4 == 0 && t.coff + t.c <= t.cstride, YL_ERR_ARG,
-                 "level %d: channels %d (expected %d) / alignment", i, t.c, no);
+        YL_CHECK(t.c == no && t.coff + t.c <= t.cstride && (no % 4 || (t.coff % 4 == 0 && t.cstride % 4 == 0)),
+                 YL_ERR_ARG, "level %d: channels %d (expected %d) / alignment", i, t.c, no);
         YL_CHECK(t.n == levels[0].n, YL_ERR_ARG, "batch mismatch at level %d", i);
         p.x[i] = reinterpret_cast<const float*>(t.data);
         p.cstride[i] = t.cstride;
@@ -142,16 +150,18 @@ extern "C" int yl_detect_decode(const yl_tensor* levels, int nl, const float* st
         p.H[i] = t.h;
         p.W[i] = t.w;
         p.tile0[i] = tiles;
-        p.anchor0[i] = A;
+        p.anchor0[i] = anchor_base + A;
         p.stride[i] = strides_host[i];
         tiles += yl::ceil_div(t.h * t.w, 32);
         A += t.h * t.w;
     }
+    YL_CHECK(anchor_base >= 0 && y_anchors >= 0 && (long long)anchor_base + A <= y_anchors, YL_ERR_ARG,
+             "anchor window [%d, %lld) outside the %d anchors of y", anchor_base, (long long)anchor_base + A, y_anchors);
     p.tile0[nl] = tiles;
     p.nl = nl;
     p.reg_max = reg_max;
     p.nc = nc;
-    p.A = A;
+    p.A = y_anchors;
     p.y = y;
     const size_t smem = (size_t)32 * (no + 1) * sizeof(float);
     YL_CHECK(smem <= 48 * 1024, YL_ERR_UNSUPPORTED, "too many head channels (%d)", no);
@@ -159,4 +169,12 @@ extern "C" int yl_detect_decode(const yl_tensor* levels, int nl, const float* st
     YL_CUDA(yl::launch_kernel(yl::detect_decode_kernel, grid, dim3(256), smem, (cudaStream_t)stream, p));
     YL_LAUNCH_OK("detect_decode_kernel");
     return YL_OK;
+}
+
+extern "C" int yl_detect_decode(const yl_tensor* levels, int nl, const float* strides_host, int reg_max, int nc,
+                                float* y, void* stream) {
+    YL_CHECK(levels && nl >= 1 && nl <= yl::kMaxLevels, YL_ERR_ARG, "1..%d levels supported", yl::kMaxLevels);
+    int A = 0;
+    for (int i = 0; i < nl; ++i) A += levels[i].h * levels[i].w;
+    return yl_detect_decode_into(levels, nl, strides_host, reg_max, nc, y, A, 0, stream);
 }

@@ -166,6 +166,8 @@ _PROTOTYPES = {
                                    C.c_void_p]),
     "yl_detect_decode": (C.c_int, [C.POINTER(Tensor), C.c_int, C.POINTER(C.c_float), C.c_int, C.c_int, C.c_void_p,
                                    C.c_void_p]),
+    "yl_detect_decode_into": (C.c_int, [C.POINTER(Tensor), C.c_int, C.POINTER(C.c_float), C.c_int, C.c_int, C.c_void_p,
+                                        C.c_int, C.c_int, C.c_void_p]),
     "yl_dfl": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "yl_nms_workspace_bytes": (C.c_size_t, [C.c_int] * 4),
     "yl_nms_batched": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_double, C.c_void_p, C.c_int,

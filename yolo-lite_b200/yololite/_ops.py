@@ -204,11 +204,17 @@ def nhwc_to_nchw(x: View, out: torch.Tensor | None = None) -> torch.Tensor:
     return out
 
 
-def detect_decode(levels: list[View], strides, reg_max: int, nc: int, y: torch.Tensor):
+def detect_decode(levels: list[View], strides, reg_max: int, nc: int, y: torch.Tensor, anchor_base: int | None = None):
+    """Decode the raw head maps `levels` into y (B, 4+nc, A) (yl_detect_decode), or, with `anchor_base`, into anchors
+    [anchor_base, anchor_base + A) of a wider y (yl_detect_decode_into)."""
     arr = (_C.Tensor * len(levels))(*[v.ct() for v in levels])
     st = (C.c_float * len(levels))(*[float(s) for s in strides])
-    _C.check(_C.load().yl_detect_decode(arr, len(levels), st, reg_max, nc, y.data_ptr(), _C.stream_ptr()),
-             "yl_detect_decode")
+    if anchor_base is None:
+        _C.check(_C.load().yl_detect_decode(arr, len(levels), st, reg_max, nc, y.data_ptr(), _C.stream_ptr()),
+                 "yl_detect_decode")
+    else:
+        _C.check(_C.load().yl_detect_decode_into(arr, len(levels), st, reg_max, nc, y.data_ptr(), y.shape[2],
+                                                 int(anchor_base), _C.stream_ptr()), "yl_detect_decode_into")
 
 
 def dfl_expectation(x: torch.Tensor, reg_max: int) -> torch.Tensor:

@@ -64,11 +64,14 @@ class Builder:
         self.lanes: list[int] = []        # lane (forked stream) of every call; 0 = the main stream
         self.deps: list[tuple] = []       # per call: indices of earlier calls whose results it reads / overwrites
         self._cur_lane = 0
+        self.lane_base = 0                # lane ids of `lane(k)` are offset by this (the members of an ensemble plan)
         self._access: dict = {}           # buffer data_ptr -> [(c0, c1, call index, is_write)]
         self.buffers: list[torch.Tensor] = []
         self.bytes = 0
         self.meta: list[dict] = []
         self.ingest: NchwInput | None = None
+        self.model_start = 0               # index of the first launch of the model being recorded (its image ingest)
+        self.n_ingest = 1                  # leading launches that read the caller's batch and stay outside the graph
         self.want_raw = True               # Detect: also write the raw head maps (module-level API)
         # single-label NMS arguments (conf, ...) of the step this plan ends with, when the Detect head may run the class
         # filter in its conv epilogues (set by BaseModel._get_plan); the head then fills `cand_ws`
@@ -108,11 +111,22 @@ class Builder:
     @contextlib.contextmanager
     def lane(self, k: int):
         """Launches emitted inside run on side lane `k` (a forked stream at graph capture)."""
-        prev, self._cur_lane = self._cur_lane, int(k)
+        prev, self._cur_lane = self._cur_lane, self.lane_base + int(k)
         try:
             yield
         finally:
             self._cur_lane = prev
+
+    @contextlib.contextmanager
+    def model(self, lane_base: int = 0):
+        """Record one model of a multi-model plan (an ensemble member): its first launch is its own image ingest, and
+        `lane(k)` inside it means lane `lane_base + k` (its main lane is `lane_base`)."""
+        self.model_start = len(self.calls)
+        self.lane_base = self._cur_lane = int(lane_base)
+        try:
+            yield
+        finally:
+            self.lane_base = self._cur_lane = 0
 
     def _track(self, idx, reads, writes):
         """RAW / WAR / WAW dependencies of call `idx` from the channel-slice access history of each buffer."""
@@ -172,8 +186,8 @@ class Builder:
             dual, out = out, out.primary
             assert not pc.depthwise and not upsample and not isinstance(x, NchwInput)
         if isinstance(x, NchwInput):
-            if (x.view is None and not self.calls and k == 3 and stride == 2 and x.c <= 4 and not pc.depthwise
-                    and res is None and not upsample and out_dtype is torch.bfloat16
+            if (x.view is None and len(self.calls) == self.model_start and k == 3 and stride == 2 and x.c <= 4
+                    and not pc.depthwise and res is None and not upsample and out_dtype is torch.bfloat16
                     and pc.co in (16, 32, 48, 64, 96)):
                 ho, wo = (x.h - 1) // 2 + 1, (x.w - 1) // 2 + 1
                 y = self._out(out, x.n, ho, wo, pc.co)
@@ -306,7 +320,7 @@ class Builder:
 
     def stem_fused(self, x: NchwInput, pc0: PackedConv, pc1: PackedConv, act0: bool, act1: bool, out=None) -> View:
         """Image ingest + the first two stride-2 3x3 convs in one launch (see yl_stem_fused)."""
-        assert x.view is None and not self.calls, "the fused stem must be the first launch of the plan"
+        assert x.view is None and len(self.calls) == self.model_start, "the fused stem must be the model's first launch"
         h0, w0 = (x.h - 1) // 2 + 1, (x.w - 1) // 2 + 1
         h1, w1 = (h0 - 1) // 2 + 1, (w0 - 1) // 2 + 1
         y = self._out(out, x.n, h1, w1, pc1.co)
@@ -367,16 +381,26 @@ class Builder:
                    flops=2 * qkv.n * heads * ntok * ntok * (key_dim + head_dim), reads=(qkv,), writes=(y,))
         return y
 
-    def detect_decode(self, levels: list[View], strides, reg_max: int, nc: int) -> torch.Tensor:
+    def detect_decode(self, levels: list[View], strides, reg_max: int, nc: int, into=None) -> torch.Tensor:
+        """`into`: None (a new (B, 4+nc, A) prediction) or (y, anchor base): write anchors [base, base + A) of the wider
+        prediction y (yl_detect_decode_into; one member of an ensemble)."""
         n = levels[0].n
         a = sum(v.h * v.w for v in levels)
-        y = torch.empty((n, 4 + nc, a), dtype=torch.float32, device=self.device)
-        self.buffers.append(y)
         arr = (_C.Tensor * len(levels))(*[v.ct() for v in levels])
         st = (C.c_float * len(levels))(*[float(s) for s in strides])
-        self._push(self.lib.yl_detect_decode, arr, len(levels), st, reg_max, nc, y.data_ptr(), keep=(arr, st),
-                   kind="detect_decode", bytes_=n * a * ((4 * reg_max + nc) * 4 + (4 + nc) * 4), reads=tuple(levels),
-                   writes=(y,))
+        bytes_ = n * a * ((4 * reg_max + nc) * 4 + (4 + nc) * 4)
+        if into is None:
+            y = torch.empty((n, 4 + nc, a), dtype=torch.float32, device=self.device)
+            self.buffers.append(y)
+            self._push(self.lib.yl_detect_decode, arr, len(levels), st, reg_max, nc, y.data_ptr(), keep=(arr, st),
+                       kind="detect_decode", bytes_=bytes_, reads=tuple(levels), writes=(y,))
+            return y
+        y, base = into
+        assert y.shape[0] == n and y.shape[1] == 4 + nc and 0 <= base and base + a <= y.shape[2], (tuple(y.shape), base, a)
+        # written range in the anchor encoding of the fused decode epilogues (2 * anchor + box | class row)
+        self._push(self.lib.yl_detect_decode_into, arr, len(levels), st, reg_max, nc, y.data_ptr(), y.shape[2], int(base),
+                   keep=(arr, st), kind="detect_decode", bytes_=bytes_, desc=f"anchors [{base}, {base + a}) of {y.shape[2]}",
+                   reads=tuple(levels), writes=((y, 2 * base, 2 * (base + a)),))
         return y
 
     def nms_begin(self, B: int, A: int, nc: int) -> torch.Tensor:
@@ -510,6 +534,17 @@ class Builder:
                 i += 1
         self.calls, self.lanes, self.deps, self.meta = calls, lanes, deps, meta
 
+    def hoist(self, first: list[int]):
+        """Move calls `first` (in this order) in front of all others: the image ingests of an ensemble's members, which
+        depend on no earlier launch, so that the plan starts with every launch that reads the caller's batch."""
+        assert all(not self.deps[i] for i in first)
+        chosen = set(first)
+        order = list(first) + [i for i in range(len(self.calls)) if i not in chosen]
+        new = {old: k for k, old in enumerate(order)}
+        self.deps = [tuple(sorted(new[d] for d in self.deps[i])) for i in order]
+        self.calls, self.lanes, self.meta = ([v[i] for i in order] for v in (self.calls, self.lanes, self.meta))
+        self._access = {}                 # call indices changed: nothing may be recorded after this
+
     def finish(self) -> "Plan":
         if self.chain_enabled:
             self._fuse_chains()
@@ -530,26 +565,31 @@ class Plan:
         self.graph: torch.cuda.CUDAGraph | None = None
         self._skip = 0
         self.n_launches = len(b.calls)
+        self.n_ingest = b.n_ingest
 
     @property
     def native_ingest(self):
-        """yl_dtypes the plan's first launch reads directly from the caller's batch: the fused stem takes fp32, fp16
-        and uint8 images; the other ingests (stem_conv, nchw_to_nhwc) read fp32 only."""
+        """yl_dtypes that every ingest launch of the plan (its first `n_ingest` calls) reads directly from the caller's
+        batch: the fused stem takes fp32, fp16 and uint8 images; the other ingests (stem_conv, nchw_to_nhwc) read fp32
+        only."""
         if not self.calls:
             return ()
-        name = self.calls[0][0].__name__
-        if name == "yl_stem_fused":
-            return (_C.YL_F32, _C.YL_F16, _C.YL_U8)
-        return (_C.YL_F32,) if name in ("yl_nchw_to_nhwc", "yl_stem_conv") else ()
+        out = (_C.YL_F32, _C.YL_F16, _C.YL_U8)
+        for fn, _, _ in self.calls[: self.n_ingest]:
+            name = fn.__name__
+            if name != "yl_stem_fused":
+                reads = (_C.YL_F32,) if name in ("yl_nchw_to_nhwc", "yl_stem_conv") else ()
+                out = tuple(d for d in out if d in reads)
+        return out
 
     def run(self, ingest_ptr: int | None = None, ingest_dtype: int = _C.YL_F32):
         """Replay.  `ingest_ptr`: device pointer of an NCHW batch (of `ingest_dtype`, one of `native_ingest`) to read
-        instead of the static input (only the first call, the image ingest, consumes it; it is never part of the CUDA
-        graph)."""
+        instead of the static input (only the first `n_ingest` calls, the image ingests, consume it; they are never part
+        of the CUDA graph)."""
         s = _C.stream_ptr()
         first = 0
         if self.graph is not None or ingest_ptr is not None:
-            for fn, args, _ in self.calls[: self._skip if self.graph is not None else 1]:
+            for fn, args, _ in self.calls[: self._skip if self.graph is not None else self.n_ingest]:
                 a = args
                 if ingest_ptr is not None and fn.__name__ in ("yl_nchw_to_nhwc", "yl_stem_conv", "yl_stem_fused"):
                     if fn.__name__ == "yl_stem_fused":
@@ -558,7 +598,7 @@ class Plan:
                         assert ingest_dtype == _C.YL_F32, "this plan's ingest kernel reads fp32 only"
                         a = (ingest_ptr,) + tuple(args[1:])
                 _C.check(fn(*a, s), fn.__name__)
-            first = self._skip if self.graph is not None else 1
+            first = self._skip if self.graph is not None else self.n_ingest
         if self.graph is not None:
             self.graph.replay()
             return

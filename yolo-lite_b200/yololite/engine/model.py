@@ -1,5 +1,6 @@
-"""YOLOLite facade (reference yololite/engine/model.py:17-146): `YOLOLite("yolo11n.pt" | "yolo11n.yaml")`,
-`model(source)`, `.predict(source, stream=False, **kwargs)`, `.val(**kwargs)`.  Training is out of scope."""
+"""YOLOLite facade (reference yololite/engine/model.py:17-146): `YOLOLite("yolo11n.pt" | "yolo11n.yaml" | [a.pt, b.pt])`
+(a list of checkpoints is a model ensemble), `model(source)`, `.predict(source, stream=False, **kwargs)`,
+`.val(**kwargs)`.  Training is out of scope."""
 from __future__ import annotations
 
 from pathlib import Path
@@ -7,7 +8,8 @@ from typing import Union
 
 import torch.nn as nn
 
-from ..nn.tasks import DetectionModel, attempt_load_one_weight, yaml_model_load
+from ..nn.tasks import _ENSEMBLE_NO_EMBED, DetectionModel, Ensemble, attempt_load_one_weight, attempt_load_weights, \
+    yaml_model_load
 from .predictor import DetectionPredictor
 
 
@@ -24,7 +26,10 @@ class YOLOLite(nn.Module):
         self.overrides = {}
         self.metrics = None
         self.task = task
-        model = str(model).strip()
+        if isinstance(model, (list, tuple)) and len(model) > 1:
+            self._load_ensemble([str(w).strip() for w in model])
+            return
+        model = str(model[0] if isinstance(model, (list, tuple)) else model).strip()
         if Path(model).suffix in {".yaml", ".yml"}:
             self._new(model, task=task, verbose=verbose)
         else:
@@ -54,6 +59,17 @@ class YOLOLite(nn.Module):
         self.overrides["task"] = self.task
         self.model_name = weights
 
+    def _load_ensemble(self, weights: list) -> None:
+        """Checkpoints loaded as one Ensemble (attempt_load_weights); overrides and ckpt_path come from member 0."""
+        self.model = attempt_load_weights(weights)
+        first = self.model[0]
+        self.task = first.args.get("task", "detect")
+        self.overrides = self.model.args = {k: v for k, v in first.args.items() if k in {"imgsz", "data", "task", "single_cls"}}
+        self.ckpt_path = first.pt_path
+        self.overrides["model"] = weights
+        self.overrides["task"] = self.task
+        self.model_name = weights
+
     def predict(self, source=None, stream: bool = False, **kwargs):
         """Same defaults as the reference (conf=0.25, batch=1, mode=predict); `save` defaults to False here
         because writing annotated images is outside the scope (the reference injects save=True, model.py:95)."""
@@ -72,7 +88,10 @@ class YOLOLite(nn.Module):
 
     def embed(self, source=None, stream: bool = False, **kwargs):
         """Image feature vectors (reference Model.embed): `predict` with `embed` defaulting to the last layer before the
-        head (22 for YOLO11; 256 values per image for yolo11n).  Yields / returns one 1-D fp32 tensor per image."""
+        head (22 for YOLO11; 256 values per image for yolo11n).  Yields / returns one 1-D fp32 tensor per image.
+        TypeError for a model ensemble (its members share no feature space)."""
+        if isinstance(self.model, Ensemble):
+            raise TypeError(_ENSEMBLE_NO_EMBED)
         if not kwargs.get("embed"):
             kwargs["embed"] = [len(self.model.model) - 2]
         return self.predict(source, stream, **kwargs)

@@ -23,7 +23,7 @@ from .. import _C
 from ..cfg import DEFAULT_CFG, get_cfg
 from ..data import LetterBox, load_inference_source
 from ..nn.autobackend import AutoBackend
-from ..nn.tasks import embed_indices
+from ..nn.tasks import _ENSEMBLE_NO_EMBED, Ensemble, embed_indices
 from ..utils import LOGGER, ops
 from ..utils.torch_utils import select_device, smart_inference_mode
 from .results import BatchDetections, Results
@@ -296,6 +296,8 @@ class DetectionPredictor:
     def stream_inference(self, source=None, model=None, *args, **kwargs):
         if not self.model:
             self.setup_model(model)
+        if self.args.embed and isinstance(self.model.model, Ensemble):
+            raise TypeError(_ENSEMBLE_NO_EMBED)
         with self._lock:
             self.setup_source(source if source is not None else self.args.source)
             self.seen, self.batch = 0, None

@@ -1,6 +1,6 @@
-"""AutoBackend (reference yololite/nn/autobackend.py:20-165): wraps a DetectionModel (in-memory module or a
-*.pt path) for the predictor: device move, `.forward(im)` -> [y, raw_list], `.warmup()`, attrs
-`stride, names, fp16, pt, device, nn_module`.  There is exactly one backend (the sm_100a kernels); `fp16`
+"""AutoBackend (reference yololite/nn/autobackend.py:20-165): wraps a DetectionModel or an Ensemble (in-memory module,
+a *.pt path, or a list of *.pt paths, which loads as an ensemble) for the predictor: device move, `.forward(im)` ->
+[y, raw_list], `.warmup()`, attrs `stride, names, fp16, pt, device, nn_module`.  There is exactly one backend (the sm_100a kernels); `fp16`
 is accepted for API compatibility — the compute type is always bf16 with fp32 accumulation."""
 from __future__ import annotations
 
@@ -22,12 +22,14 @@ class AutoBackend(nn.Module):
         if self.nn_module:
             model = weights.to(device)
         else:
-            w = str(weights[0] if isinstance(weights, list) else weights)
-            if not w.endswith(".pt"):
-                raise NotImplementedError(f"'{w}': only PyTorch *.pt checkpoints or nn.Module objects are supported")
+            ws = [str(w) for w in (weights if isinstance(weights, list) else [weights])]
+            for w in ws:
+                if not w.endswith(".pt"):
+                    raise NotImplementedError(f"'{w}': only PyTorch *.pt checkpoints or nn.Module objects are supported")
             from .tasks import attempt_load_weights
 
-            model = attempt_load_weights(w, device=device, inplace=True, fuse=fuse)
+            # a list of two or more checkpoints loads as one Ensemble (reference autobackend.py: attempt_load_weights)
+            model = attempt_load_weights(ws if len(ws) > 1 else ws[0], device=device, inplace=True, fuse=fuse)
         model = model.float().eval()
         for p in model.parameters():
             p.requires_grad = False
@@ -47,7 +49,7 @@ class AutoBackend(nn.Module):
     def forward(self, im, augment=False, visualize=False, embed=None):
         """[y, raw maps]; with `augment=True` [merged test-time-augmentation prediction, None].  With `embed=[layer
         indices]` and no `augment` (which wins, as in the reference) the per-image feature vectors of
-        `model.infer_embed`: a list of B 1-D tensors, or the tensor itself when B == 1."""
+        `model.infer_embed`: a list of B 1-D tensors, or the tensor itself when B == 1 (TypeError for an Ensemble)."""
         if visualize:
             raise NotImplementedError("visualize is not part of the inference hot path")
         if embed and not augment:

@@ -69,25 +69,41 @@ class Detect(YLModule):
             raise NotImplementedError("end2end (YOLOv10-style) heads are not part of the YOLO11 path")
 
     # ------------------------------------------------------------------ plan
+    def _fuses_decode(self) -> bool:
+        """Whether the decode runs in the epilogue of the last head convs: what the tcgen05 path needs (otherwise the
+        decode kernel runs after them)."""
+        c2, c3 = self.cv2[0][-1].in_channels, self.cv3[0][-1].in_channels
+        return (self.fuse_decode and self.reg_max == 16 and self.nc <= 256 and self.nc % 8 == 0
+                and c2 % 8 == 0 and c3 % 8 == 0)
+
+    def _fuses_filter(self, g, A: int) -> bool:
+        """Whether the class convs run the NMS class filter in their epilogue for a prediction of A anchors."""
+        import os
+
+        return (self._fuses_decode() and self.fuse_filter and getattr(g, "nms_fuse_conf", None) is not None
+                and not getattr(g, "want_raw", True) and A * self.nc < (1 << 32)
+                and os.environ.get("YL_FUSE_FILTER", "1") != "0")
+
     def _emit(self, g, feats, out=None):
-        """feats: list of nl NHWC views. Returns (y tensor (B, 4+nc, A) fp32, [raw NHWC f32 views])."""
+        """feats: list of nl NHWC views. Returns (y tensor (B, 4+nc, A) fp32, [raw NHWC f32 views]).
+
+        `out`: None, or (y, anchor base) to write anchors [base, base + A) of a wider (B, 4+nc, A_total) prediction y
+        (one member of a model ensemble).  The head then runs the class filter exactly when the caller has already begun
+        the NMS workspace of the whole prediction (`g.cand_ws`), and returns that y."""
         assert len(feats) == self.nl
         if float(self.stride.sum()) == 0.0:
             raise RuntimeError("Detect.stride is unset (it is filled in by DetectionModel)")
         nbox = 4 * self.reg_max
         want_raw = getattr(g, "want_raw", True)
-        c2, c3 = self.cv2[0][-1].in_channels, self.cv3[0][-1].in_channels
-        fuse = (self.fuse_decode and self.reg_max == 16 and self.nc <= 256 and self.nc % 8 == 0
-                and c2 % 8 == 0 and c3 % 8 == 0)          # what the tcgen05 path needs; otherwise the decode kernel
         raws = []
-        if not fuse:
+        if not self._fuses_decode():
             for i, x in enumerate(feats):
                 raw = g.alloc(x.n, x.h, x.w, self.no, dtype=torch.float32)
                 emit_any(g, self.cv2[i], x, out=raw.slice(0, nbox), out_dtype=torch.float32)
                 emit_any(g, self.cv3[i][-1], self._emit_branch(g, self.cv3[i][:-1], x), out=raw.slice(nbox, self.nc),
                          out_dtype=torch.float32)
                 raws.append(raw)
-            y = g.detect_decode(raws, [float(s) for s in self.stride], self.reg_max, self.nc)
+            y = g.detect_decode(raws, [float(s) for s in self.stride], self.reg_max, self.nc, into=out)
             return y, raws
         # fused: the last 1x1 conv of each branch decodes its logits straight into the prediction (DFL + anchors
         # + stride / sigmoid in the conv epilogue); the raw (B, H, W, no) maps are written only on request
@@ -97,15 +113,19 @@ class Detect(YLModule):
         feats = [g.mat(x) for x in feats]
         n = feats[0].n
         A = sum(x.h * x.w for x in feats)
-        y = torch.empty((n, 4 + self.nc, A), dtype=torch.float32, device=g.device)
-        g.buffers.append(y)
         import os
 
         conf = getattr(g, "nms_fuse_conf", None)
-        filt = (self.fuse_filter and conf is not None and not want_raw and self.nc <= 256
-                and A * self.nc < (1 << 32) and os.environ.get("YL_FUSE_FILTER", "1") != "0")
-        cand_ws = g.nms_begin(n, A, self.nc) if filt else None
-        a0 = 0
+        if out is None:
+            y, a0 = torch.empty((n, 4 + self.nc, A), dtype=torch.float32, device=g.device), 0
+            g.buffers.append(y)
+            filt = self._fuses_filter(g, A)
+            cand_ws = g.nms_begin(n, A, self.nc) if filt else None
+        else:
+            y, a0 = out
+            assert tuple(y.shape[:2]) == (n, 4 + self.nc) and 0 <= a0 and a0 + A <= y.shape[2], (tuple(y.shape), a0, A)
+            cand_ws = getattr(g, "cand_ws", None)
+            filt = cand_ws is not None
         for i, x in enumerate(feats):
             raw = g.alloc(x.n, x.h, x.w, self.no, dtype=torch.float32) if want_raw else None
             for j, (branch, mode, lo, cnt) in enumerate(((self.cv2[i], _C.DET_BOX, 0, nbox),

@@ -8,8 +8,9 @@ exists only at plan-build time: per input shape the whole forward is compiled in
 (optionally a CUDA graph), with skip connections and `Concat` resolved to buffer aliasing.
 Test-time augmentation (`augment=True`, reference `DetectionModel._predict_augment`) runs the plans of its three input
 shapes with two CUDA kernels around them (csrc/tta.cu).  Feature embeddings (`embed=[...]`) run a plan truncated after
-the last tapped layer that ends in one pooling kernel (csrc/embed.cu).  Training-side members (loss, criterion,
-profiling, Ensemble) are out of scope.
+the last tapped layer that ends in one pooling kernel (csrc/embed.cu).  A model ensemble (`Ensemble`, from
+`attempt_load_weights([a.pt, b.pt, ...])`) runs all its members and one NMS in one plan.  Training-side members (loss,
+criterion, profiling) are out of scope.
 """
 from __future__ import annotations
 
@@ -213,6 +214,30 @@ def fused_up_guard(layers):
     return out
 
 
+def _lru(store: dict, key, limit, dev, build):
+    """`store[key]`, made the most recently used entry (dicts keep insertion order); on a miss `build()` makes it, after
+    the least recently used entry is evicted when `limit` entries are kept.  An evicted plan's buffers / graph may still
+    be in flight on some stream, and the caching allocator would hand them to the new plan: the device is drained first
+    (rare, build-time cost)."""
+    entry = store.get(key)
+    if entry is not None:
+        store[key] = store.pop(key)
+        return entry
+    if len(store) >= max(int(limit), 1):
+        torch.cuda.synchronize(dev)
+        store.pop(next(iter(store)))
+    entry = store[key] = build()
+    return entry
+
+
+def _nms_key(conf, iou, classes, agnostic, multi_label, max_det, max_nms, max_wh) -> tuple:
+    """The NMS arguments of infer_nms as the hashable tuple of Builder.nms (part of the plan key)."""
+    if classes is not None and not isinstance(classes, (list, tuple)):
+        classes = [classes] if isinstance(classes, int) else list(classes)      # `classes=0` is legal in the reference
+    return (float(conf), float(iou), None if classes is None else tuple(int(c) for c in classes), bool(agnostic),
+            bool(multi_label), int(max_det), int(max_nms), float(max_wh))
+
+
 class BaseModel(YLModule):
     """Layer-list model executed through a cached static plan (one per input shape and device)."""
 
@@ -278,7 +303,10 @@ class BaseModel(YLModule):
 
         `embed`: sorted layer indices (embed_indices).  Only layers 0..max(embed) are recorded, and the return value is
         the list of the tapped layers' output Views (a buffer, a concat slice, a Concat's whole buffer or a fused
-        upsample's replicated copy)."""
+        upsample's replicated copy).
+
+        `out`: None, or (y, anchor base): the Detect head writes its anchors into that window of a wider prediction y
+        (Detect._emit; one member of an ensemble plan)."""
         from .._ops import View
 
         layers = list(self.model)
@@ -356,7 +384,7 @@ class BaseModel(YLModule):
                 continue
             inp = [ys[j] if j >= 0 else x for j in srcs[i]]
             if isinstance(m, Detect):
-                return m._emit(g, inp)
+                return m._emit(g, inp, out=out)
             if isinstance(m, Concat):
                 if i in cat_buf and all(place.get(j) == i for j in srcs[i]):
                     buf, chans = cat_buf[i]
@@ -386,7 +414,7 @@ class BaseModel(YLModule):
 
         if not self.fuse_stem or os.environ.get("YL_STEM_FUSE", "1") == "0" or len(layers) < 3:
             return False
-        if not isinstance(x, _plan.NchwInput) or x.view is not None or g.calls:
+        if not isinstance(x, _plan.NchwInput) or x.view is not None or len(g.calls) != g.model_start:
             return False
         l0, l1 = layers[0], layers[1]
         if type(l0) is not Conv or type(l1) is not Conv or srcs[1] != [0] or n_uses[0] != 1 or 1 in fused_up_guard(layers):
@@ -426,15 +454,8 @@ class BaseModel(YLModule):
         embeddings in place of `y` and no raw maps."""
         plans = self.__dict__.setdefault("_yl_plans", {})
         key = (tuple(shape), dev.index, bool(self.use_cuda_graph), bool(want_raw), int(slot), nms, embed)
-        entry = plans.get(key)
-        if entry is not None:
-            plans[key] = plans.pop(key)                     # most recently used last (dicts keep insertion order)
-        else:
-            if len(plans) >= max(int(self.max_plans), 1):
-                # evict the least recently used plan; its buffers / graph may still be in flight on some stream, and the
-                # caching allocator would hand them to the new plan: drain the device first (rare, build-time cost)
-                torch.cuda.synchronize(dev)
-                plans.pop(next(iter(plans)))
+
+        def build():
             with torch.cuda.device(dev):
                 g = _plan.Builder(dev)
                 g.want_raw = bool(want_raw)   # Detect writes its raw (B, H, W, no) maps only on request
@@ -451,9 +472,9 @@ class BaseModel(YLModule):
                 if self.use_cuda_graph:
                     plan.capture(skip=1)     # the image ingest stays eager so it can read the caller's tensor
                 raw_views = [r.buf.permute(0, 3, 1, 2) for r in raws]   # (B, no, H, W) views, zero-copy
-                entry = (plan, static_in, y, raw_views if post is None else post)
-            plans[key] = entry
-        return entry
+                return plan, static_in, y, raw_views if post is None else post
+
+        return _lru(plans, key, self.max_plans, dev, build)
 
     @torch.no_grad()
     def infer(self, x: torch.Tensor, want_raw: bool = False, slot: int = 0, augment: bool = False):
@@ -596,10 +617,7 @@ class BaseModel(YLModule):
         s = int(self.stride.max()) if hasattr(self, "stride") else 32
         if x.shape[2] % s or x.shape[3] % s:
             raise ValueError(f"image size {tuple(x.shape[2:])} must be a multiple of the model stride {s}")
-        if classes is not None and not isinstance(classes, (list, tuple)):
-            classes = [classes] if isinstance(classes, int) else list(classes)      # `classes=0` is legal in the reference
-        nms = (float(conf), float(iou), None if classes is None else tuple(int(c) for c in classes), bool(agnostic),
-               bool(multi_label), int(max_det), int(max_nms), float(max_wh))
+        nms = _nms_key(conf, iou, classes, agnostic, multi_label, max_det, max_nms, max_wh)
         if augment and self._augment_supported():
             from .. import _ops
 
@@ -651,6 +669,146 @@ class DetectionModel(BaseModel):
         initialize_weights(self)
 
 
+_ENSEMBLE_NO_EMBED = ("embed=[...] is not available for a model ensemble: its members have no common feature space "
+                      "(the reference's Ensemble.forward takes no embed); embed with one member instead")
+
+
+def _member_nc(m) -> int:
+    """Class count of an ensemble member: its `nc` attribute, or its Detect head's for a checkpoint's model without one."""
+    return int(m.nc) if hasattr(m, "nc") else int(m.model[-1].nc)
+
+
+class Ensemble(nn.ModuleList):
+    """Model ensemble (reference `Ensemble`, nn/tasks.py): every member runs on the same batch and their (B, 4+nc, A_k)
+    predictions are concatenated along the anchor axis in member order (anchors member-major, then as in each member),
+    so one NMS runs over the candidates of all members (the "NMS ensemble").
+
+    `names`, `nc` and `yaml` are member 0's, `stride` is that of the member with the largest `stride.max()`; members
+    must agree on the class count (AssertionError `Models differ in class counts [...]`) and the input channel count
+    (ValueError).  A member without an `nc` attribute (a checkpoint's model) counts with its Detect head's `nc`.
+
+    On the engine path one step is ONE plan: each member's image ingest (the launch it would get alone) reads the
+    caller's batch, outside the CUDA graph; the rest of every member and the NMS are one graph replay.  The members'
+    heads write straight into their anchor windows of one shared prediction, and with single-label NMS without a class
+    filter they append their candidates to one workspace that a single select launch finishes (DESIGN.md §3.7)."""
+
+    #: capture each plan into a CUDA graph; set False to debug launch by launch
+    use_cuda_graph = True
+    #: plans kept (LRU), as BaseModel.max_plans
+    max_plans = 16
+    #: return fresh tensors from forward() like the reference; engine code uses infer() and skips the copy
+    clone_outputs = True
+    #: lane ids of one member in the plan: each member's graph branches are independent of the other members'
+    _member_lanes = 16
+
+    def __init__(self, modules=None):
+        super().__init__(modules)
+        if not len(self):
+            return
+        ncs = [_member_nc(m) for m in self]
+        assert all(ncs[0] == n for n in ncs), f"Models differ in class counts {ncs}"
+        chs = [next(p for p in m.parameters() if p.dim() == 4).shape[1] for m in self]   # the first conv's input
+        if any(c != chs[0] for c in chs):
+            raise ValueError(f"ensemble members differ in input channel counts {chs}")
+        self.names, self.nc, self.yaml = self[0].names, ncs[0], self[0].yaml
+        self.stride = self[int(torch.argmax(torch.tensor([float(m.stride.max()) for m in self])))].stride
+
+    _engine_device = BaseModel._engine_device
+
+    def forward(self, x, augment=False, profile=False, visualize=False, embed=None):
+        """(torch.cat([m(x)[0] for m in self], 2), None) like the reference.  `augment=True` logs a warning and predicts
+        single-scale: the reference passes it into its members' `profile` slot and never runs TTA.  `embed` raises
+        TypeError."""
+        if embed:
+            raise TypeError(_ENSEMBLE_NO_EMBED)
+        if visualize or profile:
+            raise NotImplementedError("visualize / profile are not part of the inference hot path")
+        y, _ = self.infer(x, augment=augment)
+        return (y.clone() if self.clone_outputs else y), None
+
+    def predict(self, x, profile=False, visualize=False, augment=False, embed=None):
+        """BaseModel.predict's signature over `forward`."""
+        return self.forward(x, augment, profile, visualize, embed)
+
+    @staticmethod
+    def _single_scale(augment):
+        if augment:
+            LOGGER.warning("WARNING: test-time augmentation is not applied to model ensembles (the reference's "
+                           "Ensemble.forward never runs it); predicting single-scale.")
+
+    @torch.no_grad()
+    def infer(self, x: torch.Tensor, want_raw: bool = False, slot: int = 0, augment: bool = False):
+        """Engine entry, BaseModel.infer's signature: NCHW batch on CUDA (fp32, fp16 or uint8 image bytes) ->
+        (y (B, 4+nc, sum of the members' anchors) fp32, []).  An ensemble has no raw head maps: `want_raw` returns
+        none.  `augment=True` predicts single-scale (see forward).  y aliases a plan buffer that the next call with
+        the same shape and slot overwrites."""
+        dev = self._engine_device(x)
+        self._single_scale(augment)
+        plan, static_in, y, _ = self._get_plan(x.shape, dev, slot)
+        BaseModel._run_plan(plan, static_in, x, dev)
+        return y, []
+
+    @torch.no_grad()
+    def infer_nms(self, x: torch.Tensor, conf=0.25, iou=0.45, classes=None, agnostic=False, multi_label=False,
+                  max_det=300, max_nms=30000, max_wh=7680.0, slot: int = 0, augment: bool = False):
+        """Engine entry for a whole step, BaseModel.infer_nms's signature: the padded (dets (B, max_det, 6), counts (B,)
+        int32) of `ops.nms_padded(self.infer(x)[0], ...)`, with the NMS in the same plan / CUDA graph as the members.
+        The returned tensors alias plan buffers (same rule as BaseModel.infer_nms)."""
+        dev = self._engine_device(x)
+        self._single_scale(augment)
+        nms = _nms_key(conf, iou, classes, agnostic, multi_label, max_det, max_nms, max_wh)
+        plan, static_in, _, post = self._get_plan(x.shape, dev, slot, nms)
+        BaseModel._run_plan(plan, static_in, x, dev)
+        return post
+
+    def infer_embed(self, x, embed, slot: int = 0):
+        raise TypeError(_ENSEMBLE_NO_EMBED)
+
+    def _get_plan(self, shape, dev, slot=0, nms=None):
+        """(plan, static input, y, (dets, counts) or None) of one (shape, device, slot, NMS arguments), LRU-bounded by
+        `max_plans`."""
+        plans = self.__dict__.setdefault("_yl_plans", {})
+        key = (tuple(shape), dev.index, bool(self.use_cuda_graph), int(slot), nms)
+        return _lru(plans, key, self.max_plans, dev, lambda: self._build_plan(shape, dev, nms))
+
+    def _build_plan(self, shape, dev, nms):
+        B, _, H, W = shape
+        heads = [m.model[-1] for m in self]
+        if not all(isinstance(h, Detect) for h in heads):
+            raise NotImplementedError("ensemble members must end in a Detect head")
+        counts = [sum((H // int(s)) * (W // int(s)) for s in h.stride.tolist()) for h in heads]
+        A = sum(counts)
+        with torch.cuda.device(dev):
+            g = _plan.Builder(dev)
+            g.want_raw = False
+            if nms is not None and not nms[4] and nms[2] is None:
+                g.nms_fuse_conf = float(nms[0])
+            static_in = torch.zeros(tuple(shape), dtype=torch.float32, device=dev)
+            y = torch.empty((B, 4 + self.nc, A), dtype=torch.float32, device=dev)
+            g.buffers.append(y)
+            # the class filter runs in the heads only if every member can run it; the guards see the whole prediction
+            if g.nms_fuse_conf is not None and all(h._fuses_filter(g, A) for h in heads):
+                g.nms_begin(B, A, self.nc)
+            ingest, base = [], 0
+            for k, (m, n) in enumerate(zip(self, counts)):
+                with g.model(lane_base=k * self._member_lanes):
+                    ingest.append(g.model_start)
+                    got, _ = m._emit(g, g.input_nchw(static_in), out=(y, base))
+                assert got is y
+                base += n
+            post = g.nms(y, *nms) if nms is not None else None
+            g.hoist(ingest)
+            g.n_ingest = len(ingest)
+            plan = g.finish()
+            if self.use_cuda_graph:
+                plan.capture(skip=plan.n_ingest)     # the ingests stay eager so they can read the caller's tensor
+        return plan, static_in, y, post
+
+    def fuse(self, verbose=True):
+        """BN is folded at plan build (BaseModel.fuse): a no-op returning self."""
+        return self
+
+
 def torch_safe_load(weight):
     """torch.load of a reference/Ultralytics-format checkpoint: the pickled module classes resolve to this
     package's classes because the module paths are identical (`yololite.nn.tasks.DetectionModel`, ...)."""
@@ -682,9 +840,13 @@ def attempt_load_one_weight(weight, device=None, inplace=True, fuse=False):
 
 
 def attempt_load_weights(weights, device=None, inplace=True, fuse=False):
-    """Reference tasks.py:461-496 (single-model case; ensembles are out of scope)."""
+    """Reference tasks.py:461-496: every checkpoint of `weights` (a path or a list of paths) loaded as by
+    attempt_load_one_weight.  One checkpoint returns its model itself; two or more return an `Ensemble` of them (see
+    there: names / nc / yaml of member 0, the largest stride, class counts must agree; a member without an `nc`
+    attribute counts with its Detect head's)."""
     ws = weights if isinstance(weights, list) else [weights]
-    if len(ws) != 1:
-        raise NotImplementedError("model ensembles are out of scope")
-    model, _ = attempt_load_one_weight(ws[0], device, inplace, fuse)
-    return model
+    models = [attempt_load_one_weight(w, device, inplace, fuse)[0] for w in ws]
+    if len(models) == 1:
+        return models[0]
+    LOGGER.info(f"Ensemble created with {weights}\n")
+    return Ensemble(models)
