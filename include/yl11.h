@@ -256,6 +256,21 @@ int yl_nms_batched(const float* pred, int B, int nc, int A, float conf_thres, do
                    const int32_t* classes_dev, int n_classes, int agnostic, int multi_label, int max_det,
                    int max_nms, float max_wh, void* workspace, size_t workspace_bytes, float* out,
                    int32_t* counts, void* stream);
+/* yl_nms_batched with ground-truth priors, the `labels=` argument of ops.non_max_suppression (utils/ops.py:225-230,
+ * passed by the validator's save_hybrid): label row l of image b, (cx, cy, w, h) in pred's pixel frame
+ * label_xywh[label_offsets[b] + l] and class label_cls[...] in [0, nc) (not checked on the device), joins the
+ * image's candidates after its anchors as a row with score 1.0 at its class: it survives when conf_thres < 1 and
+ * the class filter admits it, and the max_nms cut, the class offsets and greedy NMS treat it like an anchor.
+ * An image with no anchor above conf_thres still outputs its priors.  label_offsets (B+1) int32 device array;
+ * max_labels_per_image bounds every image's count and sizes the workspace:
+ * workspace >= yl_nms_priors_workspace_bytes(B, A, nc, multi_label, max_labels_per_image), and
+ * (A + max_labels_per_image) * nc < 2^32.  label_offsets == NULL or max_labels_per_image == 0 is yl_nms_batched. */
+size_t yl_nms_priors_workspace_bytes(int B, int A, int nc, int multi_label, int max_labels_per_image);
+int yl_nms_batched_priors(const float* pred, int B, int nc, int A, float conf_thres, double iou_thres,
+                          const int32_t* classes_dev, int n_classes, int agnostic, int multi_label, int max_det,
+                          int max_nms, float max_wh, const float* label_xywh, const int32_t* label_cls,
+                          const int32_t* label_offsets, int max_labels_per_image, void* workspace,
+                          size_t workspace_bytes, float* out, int32_t* counts, void* stream);
 /* torchvision.ops.nms semantics on explicit boxes (n,4) xyxy + scores (n): keep (int64[n]) gets the kept
  * indices in descending score order, *count their number.  workspace >= yl_nms_boxes_workspace_bytes(n). */
 /* The two halves of yl_nms_batched for a step whose class filter runs inside the Detect head convs
@@ -325,6 +340,16 @@ int yl_c3k2_tail_tc(const yl_tensor* t, const yl_tensor* y, const void* wa, cons
 int yl_match_predictions(const float* dets, const int32_t* counts, int B, int max_det, const float* gt_boxes,
                          const float* gt_cls, const int32_t* gt_offsets, int max_labels_per_image,
                          const float* iou_thresholds_dev, int n_thresholds, uint8_t* tp, void* stream);
+/* ConfusionMatrix.process_batch (utils/metrics.py, called per image by the validator's update_metrics when
+ * plots=True) for a whole batch, same dets / counts / labels layout as yl_match_predictions: the detections with
+ * conf > `conf` are paired with labels of any class at box_iou > iou_thres; each detection keeps its highest-IoU
+ * pair, then each label the highest-IoU pair left (exact ties: lower label index, then lower detection index).
+ * Accumulates with integer atomics into matrix, int64[(nc+1)*(nc+1) + 1] on the device, indexed
+ * [predicted * (nc+1) + true] with nc = background: matched label [cls(det), cls(gt)], unmatched label
+ * [nc, cls(gt)], unmatched detection [cls(det), nc].  A class outside [0, nc] counts in the last element instead. */
+int yl_confusion_matrix(const float* dets, const int32_t* counts, int B, int max_det, const float* gt_boxes,
+                        const float* gt_cls, const int32_t* gt_offsets, int max_labels_per_image, int nc, float conf,
+                        float iou_thres, int64_t* matrix, void* stream);
 
 /* ---- image preprocess (the step before the path, SURVEY §8f) ---------------------------------------------- */
 /* One source image of a letterbox batch: HWC uint8 BGR on the DEVICE, `pitch` bytes per row; it is resized to

@@ -17,6 +17,10 @@
 //                               register shuffles and appends the survivors; stops at max_det survivors.
 //                               Images whose classes are provably separated by the class offsets take the
 //                               class-wise path instead (select_classwise).
+// Priors (ops.py labels=, the validator's save_hybrid): label row l of image b is the virtual anchor A + l with
+// score 1.0 at its class, its box read from the packed label buffer (MODE 2 of the select kernel).  Its keys
+// sort after every anchor key of equal score, which is the reference's row order (labels appended after the
+// anchors), so every stage downstream treats the priors exactly like anchors.
 // IoU arithmetic follows torchvision's CPU kernel operation by operation (no FMA contraction, same
 // std::max/std::min operand order, fp32 IoU compared against the double threshold).
 #include <math.h>
@@ -125,6 +129,24 @@ __global__ void __launch_bounds__(256) nms_filter_kernel(const float* __restrict
     }
 }
 
+// Candidates of the priors of image b (blockIdx.x), appended after the filter kernel's: a prior is a one-hot row (1.0
+// at its class), so both label modes give exactly one candidate (1.0, cls), kept when 1.0 > conf (checked by the
+// caller) and the class filter admits it.  Class ids are range-checked on the host.
+__global__ void nms_prior_keys_kernel(const int32_t* __restrict__ lab_cls, const int32_t* __restrict__ lab_off, int nc,
+                                      int A, const int32_t* __restrict__ classes, int n_classes, unsigned long long cap,
+                                      uint32_t* __restrict__ counts, unsigned long long* __restrict__ keys) {
+    const int b = blockIdx.x;
+    const int l0 = lab_off[b], nl = lab_off[b + 1] - l0;
+    for (int l = threadIdx.x; l < nl; l += blockDim.x) {
+        const int c = lab_cls[l0 + l];
+        bool keep = n_classes == 0;
+        for (int i = 0; i < n_classes && !keep; ++i) keep = classes[i] == c;
+        if (!keep) continue;
+        const uint32_t idx = (uint32_t)(A + l) * (uint32_t)nc + (uint32_t)c;
+        keys[(unsigned long long)b * cap + atomicAdd(&counts[b], 1u)] = ((unsigned long long)score_to_desc(1.f) << 32) | idx;
+    }
+}
+
 // keys for yl_nms_boxes: every box is a candidate
 __global__ void nms_boxes_keys_kernel(const float* __restrict__ scores, int n, unsigned long long* __restrict__ keys,
                                       uint32_t* __restrict__ counts) {
@@ -135,7 +157,7 @@ __global__ void nms_boxes_keys_kernel(const float* __restrict__ scores, int n, u
 
 // ---------------------------------------------------------------------------------------------- select
 struct SelParams {
-    const float* pred;   // MODE 0: (B, 4+nc, A) xywh+scores.  MODE 1: boxes (n,4) xyxy
+    const float* pred;   // MODE 0 / 2: (B, 4+nc, A) xywh+scores.  MODE 1: boxes (n,4) xyxy
     int nc, A;
     unsigned long long cap;
     const uint32_t* counts;
@@ -153,6 +175,8 @@ struct SelParams {
     float* out;          // MODE 0: (B, max_det, 6)
     int32_t* out_counts;
     long long* keep;     // MODE 1: int64[n]
+    const float* lab_xywh;    // MODE 2: priors (L, 4) (cx, cy, w, h); image b owns rows [lab_off[b], lab_off[b+1])
+    const int32_t* lab_off;
 };
 
 // torchvision CPU: suppressed iff inter / (area_i + area_j - inter) > thr, i = kept (earlier) box; every
@@ -184,12 +208,19 @@ __device__ __forceinline__ bool iou_suppresses(const float4 bi, float ai, const 
     return t.tie_up ? (lhs >= rhs) : (lhs > rhs);
 }
 
+// (cx, cy, w, h) of virtual anchor a >= A of image b (MODE 2): prior row a - A of the image
+__device__ __forceinline__ float4 load_prior(const SelParams& p, int b, int a) {
+    const float* q = p.lab_xywh + ((long long)__ldg(p.lab_off + b) + (a - p.A)) * 4;
+    return make_float4(__ldg(q), __ldg(q + 1), __ldg(q + 2), __ldg(q + 3));
+}
+
 // The global loads of fetch_box alone (so a caller can put other work between the loads and their use) ...
 template <int MODE>
 __device__ __forceinline__ float4 fetch_raw(const SelParams& p, int b, unsigned long long key) {
     const uint32_t idx = (uint32_t)(key & 0xffffffffull);
-    if (MODE == 0) {
+    if (MODE != 1) {
         const int a = (int)(idx / (uint32_t)p.nc);
+        if (MODE == 2 && a >= p.A) return load_prior(p, b, a);
         const float* q = p.pred + (long long)b * (4 + p.nc) * p.A + a;
         return make_float4(__ldg(q), __ldg(q + p.A), __ldg(q + 2 * (long long)p.A), __ldg(q + 3 * (long long)p.A));
     }
@@ -198,7 +229,7 @@ __device__ __forceinline__ float4 fetch_raw(const SelParams& p, int b, unsigned 
 // ... and the arithmetic: offset box (the one NMS works on) + its area, from the raw values (cx, cy, w, h | xyxy)
 template <int MODE>
 __device__ __forceinline__ void finish_box(const SelParams& p, unsigned long long key, const float4 v, float4* off, float* area) {
-    if (MODE == 0) {
+    if (MODE != 1) {
         const uint32_t idx = (uint32_t)(key & 0xffffffffull);
         const int a = (int)(idx / (uint32_t)p.nc);
         const int c = (int)(idx - (uint32_t)a * (uint32_t)p.nc);
@@ -219,12 +250,17 @@ __device__ __forceinline__ void fetch_box(const SelParams& p, int b, unsigned lo
                                           float* area, float* score, int* cls) {
     const uint32_t idx = (uint32_t)(key & 0xffffffffull);
     *score = desc_to_score((uint32_t)(key >> 32));
-    if (MODE == 0) {
+    if (MODE != 1) {
         const int a = (int)(idx / (uint32_t)p.nc);
         const int c = (int)(idx - (uint32_t)a * (uint32_t)p.nc);
-        const float* q = p.pred + (long long)b * (4 + p.nc) * p.A + a;
-        const float cx = __ldg(q), cy = __ldg(q + p.A), w = __ldg(q + 2 * (long long)p.A),
-                    h = __ldg(q + 3 * (long long)p.A);
+        float cx, cy, w, h;
+        if (MODE == 2 && a >= p.A) {
+            const float4 v = load_prior(p, b, a);
+            cx = v.x, cy = v.y, w = v.z, h = v.w;
+        } else {
+            const float* q = p.pred + (long long)b * (4 + p.nc) * p.A + a;
+            cx = __ldg(q), cy = __ldg(q + p.A), w = __ldg(q + 2 * (long long)p.A), h = __ldg(q + 3 * (long long)p.A);
+        }
         const float hw = w * 0.5f, hh = h * 0.5f;  // x[..., 2:] / 2 (exact)
         raw->x = __fsub_rn(cx, hw);
         raw->y = __fsub_rn(cy, hh);
@@ -290,6 +326,7 @@ __device__ __forceinline__ int key_bin(unsigned long long k) {
 constexpr int kCwCap = 4096;
 constexpr int kCwMaxSeg = 256;
 
+template <int MODE>
 __device__ __forceinline__ bool select_classwise(const SelParams& p, int b, int n, const unsigned long long* gkeys,
                                                  unsigned char* sm, unsigned long long* kept_keys, int* nk_out) {
     // the 128 KB key area of the general path, re-carved: sort keys | offset boxes | areas | keep flags
@@ -341,7 +378,7 @@ __device__ __forceinline__ bool select_classwise(const SelParams& p, int b, int 
         float4 rb, ob;
         float ar, sc;
         int cl;
-        fetch_box<0>(p, b, k, &rb, &ob, &ar, &sc, &cl);
+        fetch_box<MODE>(p, b, k, &rb, &ob, &ar, &sc, &cl);
         obox[i] = ob;
         oarea[i] = ar;
         if (!(rb.x == rb.x) || !(rb.z == rb.z)) bad = true;   // NaN: the extent argument does not apply
@@ -476,9 +513,11 @@ __global__ void __launch_bounds__(kSelThreads, 1) nms_select_kernel(const SelPar
     int processed = 0;   // candidates consumed in sorted order
     // per-class greedy NMS when the class offsets provably separate the classes (see select_classwise)
     bool classwise_done = false;
-    if (MODE == 0 && p.classwise && p.max_wh > 0.f && n >= 1 && n <= kCwCap && n <= p.max_nms && p.nc <= 1024 &&
-        p.A < (1 << 22) && p.kept_in_smem)
-        classwise_done = select_classwise(p, b, n, gkeys, sm, kept_keys, &nk);
+    // (anchors + priors of the image must fit the 22-bit anchor field of the regrouped keys)
+    const int n_anchors = p.A + (MODE == 2 ? p.lab_off[b + 1] - p.lab_off[b] : 0);
+    if (MODE != 1 && p.classwise && p.max_wh > 0.f && n >= 1 && n <= kCwCap && n <= p.max_nms && p.nc <= 1024 &&
+        n_anchors < (1 << 22) && p.kept_in_smem)
+        classwise_done = select_classwise<MODE>(p, b, n, gkeys, sm, kept_keys, &nk);
     __syncthreads();
     unsigned long long lo = 0;  // keys <= lo are already consumed (radix rounds)
     const bool single_round = n <= kDirectSort;
@@ -763,13 +802,13 @@ __global__ void __launch_bounds__(kSelThreads, 1) nms_select_kernel(const SelPar
     }
 
     // ---------------- emit
-    if (MODE == 0) {
+    if (MODE != 1) {
         float* o = p.out + (long long)b * p.max_det * 6;
         for (int r = tid; r < p.max_det; r += kSelThreads) {
             float4 rb = make_float4(0, 0, 0, 0), ob;
             float ar, sc = 0.f;
             int cl = 0;
-            if (r < nk) fetch_box<0>(p, b, kept_keys[r], &rb, &ob, &ar, &sc, &cl);
+            if (r < nk) fetch_box<MODE>(p, b, kept_keys[r], &rb, &ob, &ar, &sc, &cl);
             o[r * 6 + 0] = rb.x;
             o[r * 6 + 1] = rb.y;
             o[r * 6 + 2] = rb.z;
@@ -805,6 +844,7 @@ int init_nms() {
     YL_CUDA(cudaDeviceGetAttribute(&g_sel_max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
     YL_CUDA(cudaFuncSetAttribute(nms_select_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, g_sel_max_smem));
     YL_CUDA(cudaFuncSetAttribute(nms_select_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, g_sel_max_smem));
+    YL_CUDA(cudaFuncSetAttribute(nms_select_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, g_sel_max_smem));
     return YL_OK;
 }
 
@@ -860,11 +900,14 @@ __global__ void scale_boxes_kernel(float* __restrict__ dets, const int32_t* __re
 
 static int launch_select(const float* pred, int B, int nc, int A, size_t cap, const uint32_t* cand_counts,
                          const unsigned long long* keys, double iou_thres, int agnostic, int max_det, int max_nms,
-                         float max_wh, float* out, int32_t* counts, cudaStream_t s) {
+                         float max_wh, const float* lab_xywh, const int32_t* lab_off, float* out, int32_t* counts,
+                         cudaStream_t s) {
     SelParams p;
     p.pred = pred;
     p.nc = nc;
     p.A = A;
+    p.lab_xywh = lab_xywh;
+    p.lab_off = lab_off;
     p.cap = cap;
     p.counts = cand_counts;
     p.keys = keys;
@@ -883,7 +926,8 @@ static int launch_select(const float* pred, int B, int nc, int A, size_t cap, co
     p.keep = nullptr;
     const size_t smem = sel_smem_bytes(max_det, true);
     YL_CHECK((int)smem <= g_sel_max_smem, YL_ERR_UNSUPPORTED, "NMS needs %zu B shared memory (yl_init called?)", smem);
-    nms_select_kernel<0><<<B, kSelThreads, smem, s>>>(p);
+    if (lab_off) nms_select_kernel<2><<<B, kSelThreads, smem, s>>>(p);
+    else nms_select_kernel<0><<<B, kSelThreads, smem, s>>>(p);
     YL_LAUNCH_OK("nms_select_kernel");
     return YL_OK;
 }
@@ -892,31 +936,42 @@ static int launch_select(const float* pred, int B, int nc, int A, size_t cap, co
 
 extern "C" {
 
-size_t yl_nms_workspace_bytes(int B, int A, int nc, int multi_label) {
-    if (B <= 0 || A <= 0 || nc <= 0) return 0;
-    const size_t cap = multi_label ? (size_t)A * nc : (size_t)A;
+size_t yl_nms_priors_workspace_bytes(int B, int A, int nc, int multi_label, int max_labels_per_image) {
+    if (B <= 0 || A <= 0 || nc <= 0 || max_labels_per_image < 0) return 0;
+    // every prior adds at most one candidate (its own class) in either label mode
+    const size_t cap = (multi_label ? (size_t)A * nc : (size_t)A) + (size_t)max_labels_per_image;
     size_t s = yl::align_up((size_t)B * 4, 256);   // candidate counters
     s += yl::align_up((size_t)B * cap * 8, 256);   // keys
     return s;
 }
 
-int yl_nms_batched(const float* pred, int B, int nc, int A, float conf_thres, double iou_thres,
-                   const int32_t* classes_dev, int n_classes, int agnostic, int multi_label, int max_det, int max_nms,
-                   float max_wh, void* workspace, size_t workspace_bytes, float* out, int32_t* counts, void* stream) {
+size_t yl_nms_workspace_bytes(int B, int A, int nc, int multi_label) {
+    return yl_nms_priors_workspace_bytes(B, A, nc, multi_label, 0);
+}
+
+int yl_nms_batched_priors(const float* pred, int B, int nc, int A, float conf_thres, double iou_thres,
+                          const int32_t* classes_dev, int n_classes, int agnostic, int multi_label, int max_det,
+                          int max_nms, float max_wh, const float* label_xywh, const int32_t* label_cls,
+                          const int32_t* label_offsets, int max_labels_per_image, void* workspace,
+                          size_t workspace_bytes, float* out, int32_t* counts, void* stream) {
     YL_CHECK(pred && out && counts && workspace, YL_ERR_ARG, "null pointer");
     YL_CHECK(B > 0 && nc > 0 && nc <= 1024 && A > 0, YL_ERR_ARG, "bad dims B=%d nc=%d A=%d", B, nc, A);
-    YL_CHECK((long long)A * nc < (1ll << 32), YL_ERR_ARG, "A*nc must fit 32 bits");
+    YL_CHECK(max_labels_per_image >= 0, YL_ERR_ARG, "negative max_labels_per_image");
+    const int L = label_offsets ? max_labels_per_image : 0;
+    YL_CHECK(L == 0 || (label_xywh && label_cls), YL_ERR_ARG, "label_xywh / label_cls is NULL");
+    YL_CHECK((long long)(A + (long long)L) * nc < (1ll << 32), YL_ERR_ARG, "(A + max_labels_per_image)*nc must fit 32 bits");
     YL_CHECK(max_det > 0 && max_det <= 1024, YL_ERR_ARG, "max_det must be in [1,1024]");
     YL_CHECK(max_nms > 0, YL_ERR_ARG, "max_nms must be positive");
     YL_CHECK(conf_thres >= 0.f && conf_thres <= 1.f && iou_thres >= 0. && iou_thres <= 1., YL_ERR_ARG,
              "thresholds must be in [0,1]");
     YL_CHECK(n_classes == 0 || classes_dev, YL_ERR_ARG, "classes_dev is NULL");
-    const size_t need = yl_nms_workspace_bytes(B, A, nc, multi_label);
+    const size_t need = yl_nms_priors_workspace_bytes(B, A, nc, multi_label, L);
     YL_CHECK(workspace_bytes >= need, YL_ERR_WORKSPACE, "NMS workspace too small: %zu < %zu", workspace_bytes, need);
     cudaStream_t s = (cudaStream_t)stream;
     multi_label = multi_label && nc > 1;
+    const int32_t* lab_off = L > 0 ? label_offsets : nullptr;   // no priors: the plain path, launch for launch
 
-    const size_t cap = multi_label ? (size_t)A * nc : (size_t)A;
+    const size_t cap = (multi_label ? (size_t)A * nc : (size_t)A) + (size_t)L;
     uint32_t* cand_counts = reinterpret_cast<uint32_t*>(workspace);
     unsigned long long* keys =
         reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(workspace) + yl::align_up((size_t)B * 4, 256));
@@ -935,9 +990,22 @@ int yl_nms_batched(const float* pred, int B, int nc, int A, float conf_thres, do
 #undef YL_FILTER
     }
     YL_LAUNCH_OK("nms_filter_kernel");
+    if (lab_off && 1.f > conf_thres) {
+        yl::nms_prior_keys_kernel<<<B, 128, 0, s>>>(label_cls, lab_off, nc, A, classes_dev, n_classes,
+                                                    (unsigned long long)cap, cand_counts, keys);
+        YL_LAUNCH_OK("nms_prior_keys_kernel");
+    }
 
-    return yl::launch_select(pred, B, nc, A, cap, cand_counts, keys, iou_thres, agnostic, max_det, max_nms, max_wh, out,
-                             counts, s);
+    return yl::launch_select(pred, B, nc, A, cap, cand_counts, keys, iou_thres, agnostic, max_det, max_nms, max_wh,
+                             label_xywh, lab_off, out, counts, s);
+}
+
+int yl_nms_batched(const float* pred, int B, int nc, int A, float conf_thres, double iou_thres,
+                   const int32_t* classes_dev, int n_classes, int agnostic, int multi_label, int max_det, int max_nms,
+                   float max_wh, void* workspace, size_t workspace_bytes, float* out, int32_t* counts, void* stream) {
+    return yl_nms_batched_priors(pred, B, nc, A, conf_thres, iou_thres, classes_dev, n_classes, agnostic, multi_label,
+                                 max_det, max_nms, max_wh, nullptr, nullptr, nullptr, 0, workspace, workspace_bytes, out,
+                                 counts, stream);
 }
 
 int yl_debug_nms_phases(long long* device_buf) {
@@ -963,7 +1031,7 @@ int yl_nms_select(const float* pred, int B, int nc, int A, double iou_thres, int
     unsigned long long* keys =
         reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(workspace) + yl::align_up((size_t)B * 4, 256));
     return yl::launch_select(pred, B, nc, A, (size_t)A, cand_counts, keys, iou_thres, agnostic, max_det, max_nms, max_wh,
-                             out, counts, (cudaStream_t)stream);
+                             nullptr, nullptr, out, counts, (cudaStream_t)stream);
 }
 
 size_t yl_nms_boxes_workspace_bytes(int n) {
@@ -997,6 +1065,8 @@ int yl_nms_boxes(const float* boxes, const float* scores, int n, double iou_thre
     p.pred = boxes;
     p.nc = 1;
     p.A = n;
+    p.lab_xywh = nullptr;
+    p.lab_off = nullptr;
     p.cap = (unsigned long long)n;
     p.counts = cand_counts;
     p.keys = keys;

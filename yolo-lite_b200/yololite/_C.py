@@ -173,6 +173,11 @@ _PROTOTYPES = {
     "yl_nms_batched": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_double, C.c_void_p, C.c_int,
                                  C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p, C.c_size_t, C.c_void_p,
                                  C.c_void_p, C.c_void_p]),
+    "yl_nms_priors_workspace_bytes": (C.c_size_t, [C.c_int] * 5),
+    "yl_nms_batched_priors": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_double, C.c_void_p,
+                                        C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
+                                        C.c_void_p]),
     "yl_nms_begin": (C.c_int, [C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
     "yl_debug_nms_phases": (C.c_int, [C.c_void_p]),
     "yl_nms_select": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, C.c_int, C.c_float,
@@ -193,6 +198,8 @@ _PROTOTYPES = {
                                C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "yl_match_predictions": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                        C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "yl_confusion_matrix": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_int, C.c_int, C.c_float, C.c_float, C.c_void_p, C.c_void_p]),
     "yl_letterbox_u8": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "yl_tta_scale_img": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(TtaCanvas),
                                    C.c_void_p]),

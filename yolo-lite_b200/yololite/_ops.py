@@ -244,14 +244,28 @@ class NmsWorkspace:
 
 
 def nms_batched(pred: torch.Tensor, conf: float, iou: float, classes=None, agnostic=False, multi_label=False,
-                max_det=300, max_nms=30000, max_wh=7680.0, out=None, counts=None):
+                max_det=300, max_nms=30000, max_wh=7680.0, out=None, counts=None, labels=None):
     """pred (B, 4+nc, A) fp32 contiguous CUDA -> (dets (B, max_det, 6) fp32, counts (B,) int32), all async.
-    `classes`: None, a sequence of class ids, or a contiguous int32 tensor of them on pred's device."""
+    `classes`: None, a sequence of class ids, or a contiguous int32 tensor of them on pred's device.
+    `labels`: None or ground-truth priors packed as (xywh (L, 4) fp32, cls (L,) int32, both on pred's device, and the
+    B + 1 host ints `offsets`: image b owns rows [offsets[b], offsets[b+1])); class ids must already be in [0, nc)."""
     lib = _C.init(pred.device)
     assert pred.is_cuda and pred.dtype == torch.float32 and pred.is_contiguous() and pred.dim() == 3
     B, C4, A = pred.shape
     nc = C4 - 4
-    ws_bytes = lib.yl_nms_workspace_bytes(B, A, nc, int(multi_label))
+    lab_xywh = lab_cls = lab_off = None
+    max_l = 0
+    if labels is not None:
+        lab_xywh, lab_cls, offsets = labels
+        offsets = [int(o) for o in offsets]
+        assert len(offsets) == B + 1 and offsets[0] == 0, "labels: offsets must be B + 1 ints starting at 0"
+        max_l = max(e - s for s, e in zip(offsets[:-1], offsets[1:]))
+        assert max_l >= 0 and lab_xywh.shape == (offsets[-1], 4) and lab_cls.shape == (offsets[-1],)
+        assert lab_xywh.dtype == torch.float32 and lab_cls.dtype == torch.int32
+        assert lab_xywh.device == pred.device and lab_cls.device == pred.device
+        lab_xywh, lab_cls = lab_xywh.contiguous(), lab_cls.contiguous()
+        lab_off = torch.as_tensor(offsets, dtype=torch.int32).to(pred.device)
+    ws_bytes = lib.yl_nms_priors_workspace_bytes(B, A, nc, int(multi_label), max_l)
     ws = NmsWorkspace.get(ws_bytes, pred.device)
     if out is None:
         out = torch.empty((B, max_det, 6), dtype=torch.float32, device=pred.device)
@@ -262,10 +276,11 @@ def nms_batched(pred: torch.Tensor, conf: float, iou: float, classes=None, agnos
         cls_t = classes
     elif classes is not None:
         cls_t = torch.as_tensor(list(classes), dtype=torch.int32).to(pred.device)
-    _C.check(lib.yl_nms_batched(pred.data_ptr(), B, nc, A, float(conf), float(iou), _ptr(cls_t),
-                                0 if cls_t is None else cls_t.numel(), int(agnostic), int(multi_label), int(max_det),
-                                int(max_nms), float(max_wh), ws.data_ptr(), ws.numel(), out.data_ptr(),
-                                counts.data_ptr(), _C.stream_ptr()), "yl_nms_batched")
+    _C.check(lib.yl_nms_batched_priors(pred.data_ptr(), B, nc, A, float(conf), float(iou), _ptr(cls_t),
+                                       0 if cls_t is None else cls_t.numel(), int(agnostic), int(multi_label),
+                                       int(max_det), int(max_nms), float(max_wh), _ptr(lab_xywh), _ptr(lab_cls),
+                                       _ptr(lab_off), max_l, ws.data_ptr(), ws.numel(), out.data_ptr(),
+                                       counts.data_ptr(), _C.stream_ptr()), "yl_nms_batched_priors")
     return out, counts
 
 

@@ -6,6 +6,11 @@ iou 0.7, max_det 300, multi_label NMS) and the `stats` / `DetMetrics` outputs.  
 label preparation and `box_iou + match_predictions` (a per-image torch/numpy loop in the reference, :313-360) run
 batched on the GPU (`yl_scale_boxes`, `yl_match_predictions`); one host read per batch.
 
+Two switches of the reference are kept: `save_hybrid=True` passes each image's ground-truth labels to NMS as priors
+(hybrid metrics, inflated by construction), `plots=True` accumulates a `ConfusionMatrix` (`yl_confusion_matrix`, one
+launch per batch), exposed as `validator.confusion_matrix` and `metrics.confusion_matrix`.  Neither launches or
+allocates anything while it is off.
+
 Dataset construction (data/build.py, data/dataset.py, augmentations, caching) is training-side I/O and out of scope:
 pass `dataloader=` (any iterable of batch dicts) instead of a dataset yaml."""
 from __future__ import annotations
@@ -16,7 +21,7 @@ import torch
 from .. import _C
 from ..cfg import DEFAULT_CFG, get_cfg
 from ..utils import LOGGER, ops
-from ..utils.metrics import DetMetrics, match_predictions_batched
+from ..utils.metrics import ConfusionMatrix, DetMetrics, match_predictions_batched
 from ..utils.torch_utils import select_device, smart_inference_mode
 
 
@@ -34,10 +39,24 @@ class DetectionValidator:
         self.metrics = DetMetrics()
         self.stats = None
         self.speed = {"preprocess": 0.0, "inference": 0.0, "loss": 0.0, "postprocess": 0.0}
+        self.confusion_matrix = None
+        self.lb = None              # save_hybrid priors of the current batch (packed for ops.nms_padded)
+        self._layout = None         # (label order, offsets) of the current batch
+        if self.args.save_hybrid:   # reference DetectionValidator.__init__
+            LOGGER.warning("WARNING 'save_hybrid=True' will append ground truth to predictions for autolabelling.\n"
+                           "WARNING 'save_hybrid=True' will cause incorrect mAP.\n")
 
     # ------------------------------------------------------------------ stages
     def preprocess(self, batch):
-        """uint8 / float image batch -> float [0, 1] on the device (reference :262-266 divides by 255)."""
+        """uint8 / float image batch -> float [0, 1] on the device (reference :262-266 divides by 255).  With
+        save_hybrid, the priors: each image's labels in their original order, boxes `bboxes * (w, h, w, h)` of the
+        network input, built where the loader left them (on the host for a CPU loader, so no device read)."""
+        self._layout = None
+        if self.args.save_hybrid:
+            h, w = batch["img"].shape[2:]
+            order, offsets = self._label_layout(batch)
+            bboxes = batch["bboxes"].view(-1, 4)[order].float()
+            self.lb = (bboxes * torch.tensor((w, h, w, h), device=bboxes.device), batch["cls"].view(-1)[order], offsets)
         img = batch["img"].to(self.device, non_blocking=True)
         batch["img"] = img.float() / 255 if img.dtype == torch.uint8 else img.float()
         for k in ("batch_idx", "cls", "bboxes"):
@@ -47,7 +66,8 @@ class DetectionValidator:
     def postprocess(self, preds):
         """Batched NMS with the validator's settings (multi_label, reference :280-290); device-resident."""
         a = self.args
-        return ops.nms_padded(preds, a.conf, a.iou, None, a.single_cls or a.agnostic_nms, True, a.max_det)
+        return ops.nms_padded(preds, a.conf, a.iou, None, a.single_cls or a.agnostic_nms, True, a.max_det,
+                              labels=self.lb if a.save_hybrid else None)
 
     def init_metrics(self, model):
         self.names = model.names
@@ -55,18 +75,24 @@ class DetectionValidator:
         self.metrics = DetMetrics(names=self.names)
         self.seen = 0
         self.stats = dict(tp=[], conf=[], pred_cls=[], target_cls=[], target_img=[])
+        self.confusion_matrix = ConfusionMatrix(nc=self.nc, conf=self.args.conf) if self.args.plots else None
+
+    def _label_layout(self, batch):
+        """Stable image-major order of the batch's labels and the B + 1 per-image offsets, once per batch."""
+        if self._layout is None:
+            bi = batch["batch_idx"].long().view(-1)
+            counts = torch.bincount(bi, minlength=batch["img"].shape[0])
+            self._layout = (torch.argsort(bi, stable=True), [0] + torch.cumsum(counts, 0).tolist())
+        return self._layout
 
     def _labels_native(self, batch):
         """Labels of the whole batch in original-image pixels (reference _prepare_batch :234-246), image-major."""
         B = batch["img"].shape[0]
         h, w = batch["img"].shape[2:]
-        bi = batch["batch_idx"].long().view(-1)
-        order = torch.argsort(bi, stable=True)
-        bi = bi[order]
+        order, offsets = self._label_layout(batch)
+        order = order.to(self.device)
         cls = batch["cls"].view(-1)[order].float()
         box = ops.xywh2xyxy(batch["bboxes"].view(-1, 4)[order].float()) * torch.tensor([w, h, w, h], device=self.device)
-        counts = torch.bincount(bi, minlength=B)
-        offsets = [0] + torch.cumsum(counts, 0).tolist()
         for si in range(B):                               # labels are few: the reference's own helper, per image
             s, e = offsets[si], offsets[si + 1]
             if e > s:
@@ -91,6 +117,8 @@ class DetectionValidator:
                  "yl_scale_boxes")
         gt_box, gt_cls, offsets = self._labels_native(batch)
         tp = match_predictions_batched(predn, counts, gt_box, gt_cls, offsets, self.iouv)
+        if self.confusion_matrix is not None:
+            self.confusion_matrix.process_batched(predn, counts, gt_box, gt_cls, offsets)
         n = counts.tolist()                               # the one host read of the batch
         for si in range(B):
             self.seen += 1
@@ -116,6 +144,9 @@ class DetectionValidator:
 
     def finalize_metrics(self):
         self.metrics.speed = self.speed
+        if self.confusion_matrix is not None:
+            self.confusion_matrix.matrix   # the one host read of the accumulated counts
+        self.metrics.confusion_matrix = self.confusion_matrix
 
     def print_results(self):
         pf = "%22s" + "%11i" * 2 + "%11.3g" * len(self.metrics.keys)

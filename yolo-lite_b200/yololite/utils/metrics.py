@@ -1,16 +1,20 @@
-"""Detection metrics of the validator (reference yololite/utils/metrics.py: box_iou :51-70, compute_ap :445-474,
-ap_per_class :477-564, Metric :567-736, DetMetrics :739-840; engine/validator.py match_predictions :195-233).
+"""Detection metrics of the validator (reference yololite/utils/metrics.py: box_iou :51-70, ConfusionMatrix,
+compute_ap :445-474, ap_per_class :477-564, Metric :567-736, DetMetrics :739-840; engine/validator.py
+match_predictions :195-233).
 
 `box_iou` + `match_predictions` — the per-image torch/numpy loop of the reference's `update_metrics` — run as ONE
 CUDA kernel over the whole batch (`match_predictions_batched`, csrc/metrics.cu) on the padded NMS output;
-`ap_per_class` stays numpy on the host (it runs once per validation, on a few thousand rows).  Plots, confusion
-matrix and JSON export are visualisation / I-O and out of scope."""
+`ap_per_class` stays numpy on the host (it runs once per validation, on a few thousand rows).  The validator's
+`ConfusionMatrix` (plots=True) is a metric too: its per-image `process_batch` runs as one CUDA kernel per batch
+(`yl_confusion_matrix`) into a device-resident integer matrix that the host reads once.  Drawing plots and JSON
+export are visualisation / I-O and out of scope."""
 from __future__ import annotations
 
 import numpy as np
 import torch
 
-__all__ = ("box_iou", "match_predictions_batched", "compute_ap", "ap_per_class", "Metric", "DetMetrics", "smooth")
+__all__ = ("box_iou", "match_predictions_batched", "ConfusionMatrix", "compute_ap", "ap_per_class", "Metric",
+           "DetMetrics", "smooth")
 
 
 def box_iou(box1: torch.Tensor, box2: torch.Tensor, eps: float = 1e-7) -> torch.Tensor:
@@ -49,6 +53,87 @@ def match_predictions_batched(dets: torch.Tensor, counts: torch.Tensor, gt_boxes
                                       gtc.data_ptr() if gtc.numel() else None, offs.data_ptr(), max_l, thr.data_ptr(),
                                       thr.numel(), tp.data_ptr(), _C.stream_ptr()), "yl_match_predictions")
     return tp.bool()
+
+
+class ConfusionMatrix:
+    """Detection confusion matrix (reference utils/metrics.py ConfusionMatrix, task "detect").
+
+    `matrix` is (nc+1, nc+1) float64 indexed [predicted, true]; index nc is background.  Detections count when
+    conf > `conf` (0.25 when given None or the validator's default 0.001), pairs when IoU > `iou_thres`.  Counts
+    accumulate on the GPU (`process_batch` per image, `process_batched` per validator batch) and are folded into
+    `matrix` on the first read after them."""
+
+    def __init__(self, nc, conf=0.25, iou_thres=0.45, task="detect"):
+        if task != "detect":
+            raise NotImplementedError(f"ConfusionMatrix task {task!r}: only detection is on the GPU path")
+        self.task = task
+        self.nc = nc
+        self.conf = 0.25 if conf in {None, 0.001} else conf
+        self.iou_thres = iou_thres
+        self._matrix = np.zeros((nc + 1, nc + 1))
+        self._counts = None   # device int64[(nc+1)^2 + 1] accumulator; the last element counts out-of-range classes
+
+    @property
+    def matrix(self) -> np.ndarray:
+        if self._counts is not None:   # the one host read of the accumulated batches
+            c = self._counts.cpu().numpy()
+            self._counts = None
+            if c[-1]:
+                raise ValueError(f"ConfusionMatrix: {int(c[-1])} class ids outside [0, {self.nc}]")
+            self._matrix += c[:-1].reshape(self.nc + 1, self.nc + 1)
+        return self._matrix
+
+    @matrix.setter
+    def matrix(self, value):
+        self._counts = None
+        self._matrix = np.asarray(value, dtype=np.float64)
+
+    def process_batched(self, dets, counts, gt_boxes, gt_cls, gt_offsets):
+        """A whole batch in one launch, the layout of `match_predictions_batched`: dets (B, max_det, 6) + counts (B,)
+        on the GPU (boxes in the labels' space), gt_boxes (L, 4) xyxy, gt_cls (L,), gt_offsets B + 1 host ints."""
+        from .. import _C
+
+        if not dets.is_cuda:
+            raise RuntimeError("ConfusionMatrix runs on CUDA (sm_100) only; there is no CPU fallback")
+        lib = _C.init(dets.device)
+        dev = dets.device
+        B, max_det, _ = dets.shape
+        offs = [int(o) for o in gt_offsets]
+        assert len(offs) == B + 1
+        max_l = max(e - s for s, e in zip(offs[:-1], offs[1:]))
+        offs_t = torch.as_tensor(offs, dtype=torch.int32).to(dev)
+        gtb = gt_boxes.to(dev, torch.float32).contiguous().view(-1, 4)
+        gtc = gt_cls.to(dev, torch.float32).contiguous().view(-1)
+        d = dets if (dets.dtype == torch.float32 and dets.is_contiguous()) else dets.float().contiguous()
+        c = counts.to(dev, torch.int32).contiguous()
+        if self._counts is None:
+            self._counts = torch.zeros((self.nc + 1) ** 2 + 1, dtype=torch.int64, device=dev)
+        _C.check(lib.yl_confusion_matrix(d.data_ptr(), c.data_ptr(), B, max_det, gtb.data_ptr() if gtb.numel() else None,
+                                         gtc.data_ptr() if gtc.numel() else None, offs_t.data_ptr(), max_l, self.nc,
+                                         float(self.conf), float(self.iou_thres), self._counts.data_ptr(),
+                                         _C.stream_ptr()), "yl_confusion_matrix")
+
+    def process_batch(self, detections, gt_bboxes, gt_cls):
+        """One image, the reference's signature: detections (N, 6) [x1, y1, x2, y2, conf, cls] or None, gt_bboxes
+        (M, 4) xyxy, gt_cls (M,)."""
+        dev = gt_bboxes.device if detections is None else detections.device
+        n = 0 if detections is None else detections.shape[0]
+        dets = torch.zeros((1, max(n, 1), 6), dtype=torch.float32, device=dev)
+        if n:
+            dets[0, :n] = detections[:, :6].float()
+        counts = torch.tensor([n], dtype=torch.int32).to(dev)
+        self.process_batched(dets, counts, gt_bboxes, gt_cls, [0, gt_cls.shape[0]])
+
+    def tp_fp(self):
+        """True and false positives per class (background excluded)."""
+        tp = self.matrix.diagonal()
+        fp = self.matrix.sum(1) - tp
+        return tp[:-1], fp[:-1]
+
+    def plot(self, normalize=True, save_dir="", names=(), on_plot=None):
+        from . import LOGGER
+
+        LOGGER.info("ConfusionMatrix.plot: drawing plots is outside yololite's scope; read `.matrix` instead")
 
 
 def smooth(y, f=0.05):
@@ -166,6 +251,7 @@ class DetMetrics:
         self.box = Metric()
         self.speed = {"preprocess": 0.0, "inference": 0.0, "loss": 0.0, "postprocess": 0.0}
         self.task = "detect"
+        self.confusion_matrix = None   # the validator's ConfusionMatrix when it ran with plots=True
 
     def process(self, tp, conf, pred_cls, target_cls):
         results = ap_per_class(tp, conf, pred_cls, target_cls)[2:]

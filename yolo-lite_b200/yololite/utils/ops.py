@@ -6,6 +6,8 @@ per-image Python loop, boolean-index compaction (host syncs) and torchvision.ops
 batched CUDA kernels (csrc/nms.cu) that are bit-exact against the reference's CPU arithmetic; the only host
 synchronisation is one read of the (B,) counts at the end.  There is no wall-clock early exit
 (`max_time_img` is accepted and ignored: the reference silently drops images when it fires, ops.py:269-271).
+Ground-truth priors (`labels=`, ops.py:225-230) join each image's candidates after its anchors inside the same
+two kernels (`yl_nms_batched_priors`).
 """
 from __future__ import annotations
 
@@ -116,22 +118,54 @@ def convert_torch2numpy_batch(batch: torch.Tensor) -> np.ndarray:
     return (batch.permute(0, 2, 3, 1).contiguous() * 255).clamp(0, 255).to(torch.uint8).cpu().numpy()
 
 
+def pack_priors(labels, device=None):
+    """The reference's `labels` argument (B tensors (n_i, 5): cls, cx, cy, w, h) -> the packed priors of
+    `nms_padded`: (xywh (L, 4), cls (L,), offsets: B + 1 ints), on the labels' own device unless `device` is given."""
+    offsets = [0]
+    for lb in labels:
+        offsets.append(offsets[-1] + len(lb))
+    rows = [lb.reshape(-1, 5) for lb in labels]
+    lb = torch.cat([r.to(device) if device is not None else r for r in rows], 0) if rows else torch.zeros((0, 5))
+    return lb[:, 1:5], lb[:, 0], offsets
+
+
+def _check_priors(labels, nc):
+    """Validate packed priors; returns them as (xywh, int64 cls, offsets).  The range test runs where the class ids
+    are: free on the host, one read for device tensors."""
+    xywh, cls, offsets = labels
+    offsets = [int(o) for o in offsets]
+    if xywh.shape != (offsets[-1], 4) or cls.reshape(-1).shape != (offsets[-1],):
+        raise ValueError(f"labels: {tuple(xywh.shape)} boxes and {tuple(cls.shape)} classes for {offsets[-1]} priors")
+    cls = cls.reshape(-1).long()   # lb[:, 0].long() of the reference
+    if cls.numel() and bool(((cls < 0) | (cls >= nc)).any()):
+        bad = cls[(cls < 0) | (cls >= nc)][0].item()
+        raise ValueError(f"labels: class id {bad} is outside [0, {nc})")
+    return xywh, cls, offsets
+
+
 def nms_padded(prediction, conf_thres=0.25, iou_thres=0.45, classes=None, agnostic=False, multi_label=False,
-               max_det=300, nc=0, max_nms=30000, max_wh=7680, out=None, counts=None):
+               max_det=300, nc=0, max_nms=30000, max_wh=7680, out=None, counts=None, labels=None):
     """Device-resident NMS: (B, 4+nc, A) -> (dets (B, max_det, 6) fp32, counts (B,) int32), fully async.
 
+    `labels`: None or ground-truth priors packed as `pack_priors` returns them (boxes in the prediction's pixel frame;
+    CPU or CUDA); a class id outside [0, nc) raises ValueError.
     This is what the engine uses; `non_max_suppression` below turns it into the reference's list layout."""
     if isinstance(prediction, (list, tuple)):
         prediction = prediction[0]
+    nc = nc or (prediction.shape[1] - 4)
+    if labels is not None:
+        labels = _check_priors(labels, nc)
     if not prediction.is_cuda:
         raise RuntimeError("yololite NMS runs on CUDA (sm_100) only; there is no CPU fallback")
-    nc = nc or (prediction.shape[1] - 4)
     if prediction.shape[1] != 4 + nc:
         raise NotImplementedError("mask coefficients (nm > 0) are outside the detection path")
     pred = prediction if (prediction.dtype == torch.float32 and prediction.is_contiguous()) else \
         prediction.float().contiguous()
+    if labels is not None:
+        xywh, cls, offsets = labels
+        labels = (xywh.to(pred.device, torch.float32), cls.to(pred.device, torch.int32), offsets)
     return _ops.nms_batched(pred, conf_thres, iou_thres, classes, agnostic, multi_label, max_det, max_nms, max_wh,
-                            out=out, counts=counts)
+                            out=out, counts=counts, labels=labels)
 
 
 def non_max_suppression(
@@ -151,23 +185,28 @@ def non_max_suppression(
     rotated=False,
 ):
     """Drop-in for the reference's non_max_suppression: returns a list (one per image) of (n, 6) tensors
-    [x1, y1, x2, y2, confidence, class] sorted by descending confidence."""
+    [x1, y1, x2, y2, confidence, class] sorted by descending confidence.  `labels`: the reference's autolabel priors,
+    one (n_i, 5) tensor [cls, cx, cy, w, h] per image (CPU or CUDA), appended to the image's candidates with score
+    1.0; a class id outside [0, nc) raises ValueError (the reference fails with an IndexError there)."""
     assert 0 <= conf_thres <= 1, f"Invalid Confidence threshold {conf_thres}, valid values are between 0.0 and 1.0"
     assert 0 <= iou_thres <= 1, f"Invalid IoU {iou_thres}, valid values are between 0.0 and 1.0"
     if isinstance(prediction, (list, tuple)):
         prediction = prediction[0]
     if rotated:
         raise NotImplementedError("rotated boxes (OBB) are outside the detection path")
-    if labels:
-        raise NotImplementedError("autolabel priors (`labels`, validator save_hybrid) are outside the hot path")
     if prediction.shape[-1] == 6:  # end2end layout (B, N, 6): plain confidence filter, as in the reference
         output = [p[p[:, 4] > conf_thres][:max_det] for p in prediction]
         if classes is not None:
             cl = torch.tensor(classes, device=prediction.device)
             output = [p[(p[:, 5:6] == cl).any(1)] for p in output]
         return output
+    priors = None
+    if labels is not None and len(labels):
+        if len(labels) != prediction.shape[0]:
+            raise ValueError(f"labels: {len(labels)} entries for a batch of {prediction.shape[0]} images")
+        priors = pack_priors(labels)
     dets, counts = nms_padded(prediction, conf_thres, iou_thres, classes, agnostic, multi_label, max_det, nc,
-                              max_nms, max_wh)
+                              max_nms, max_wh, labels=priors)
     if in_place and prediction.dtype == torch.float32 and prediction.is_contiguous():
         # observable side effect of the reference (ops.py:213): caller's boxes become xyxy
         from .. import _C
