@@ -414,6 +414,57 @@ typedef struct yl_embed_tap {
 int yl_embed_pool(const yl_embed_tap* taps, int n_taps, int B, int D, float* out, void* workspace, size_t* workspace_bytes,
                   void* stream);
 
+/* ---- COCO bbox evaluation (the validator's save_json=True; pycocotools 2.0.x COCOeval, iouType="bbox") --------- */
+/* The evaluated set in flat DEVICE arrays.  Pairs are the (category, image) pairs with at least one gt or dt, in
+ * category-major order with image ranks (ascending image ids) ascending inside a category; gts and dts are CSR over
+ * the pairs.  A pair's gts are in annotation-file order; its dts are its kept results: ordered by descending score with
+ * ties in results-list order (np.argsort(-score, kind="mergesort")) and cut to maxDets[-1].  Every value is finite. */
+typedef struct yl_cocoeval_set {
+    int32_t n_pairs, n_cats, n_slots;  /* n_slots: kept dts in all */
+    int32_t max_gt, max_dt;       /* largest gt group and largest kept dt group of one pair */
+    const int32_t* pair_cat;      /* [n_pairs] category index */
+    const int32_t* gt_off;        /* [n_pairs + 1] */
+    const double* gt_bbox;        /* [n_gt][4] x, y, w, h */
+    const double* gt_area;        /* [n_gt] the annotation's area (not w * h) */
+    const uint8_t* gt_iscrowd;    /* [n_gt] */
+    const int64_t* gt_id;         /* [n_gt] */
+    const int32_t* slot_off;      /* [n_pairs + 1] CSR of the kept dts */
+    const double* dt_bbox;        /* [n_slots][4] */
+    const double* dt_score;       /* [n_slots] */
+    const double* dt_area;        /* [n_slots] w * h (COCO.loadRes) */
+    const int64_t* dt_id;         /* [n_slots] */
+} yl_cocoeval_set;
+/* COCOeval.params, DEVICE arrays: iouThrs[T], recThrs[R], areaRng[A][2] (A <= 16), maxDets[M] ascending. */
+typedef struct yl_cocoeval_params {
+    const double* iou_thrs;
+    const double* rec_thrs;
+    const double* area_rng;
+    const int32_t* max_dets;
+    int32_t T, R, A, M;
+} yl_cocoeval_params;
+/* Outputs of yl_cocoeval_evaluate per kept dt slot: an int64 key whose ascending order is descending score, its rank in
+ * its pair, and flags[A][T][n_slots] with bit 0 = dtMatches != 0, bit 1 = dtIgnore; npig[K][A]: non-ignored gts per
+ * category and area range. */
+typedef struct yl_cocoeval_slots {
+    int64_t* key;
+    int32_t* rank;
+    uint8_t* flags;
+    int32_t* npig;
+} yl_cocoeval_slots;
+/* COCOeval.computeIoU + COCOeval.evaluateImg (maxDet = maxDets[-1]) of every pair in ONE launch: maskApi bbIou in
+ * fp64, the greedy match with its quirks (equal IoU: the later gt in the ignore-sorted order wins; crowd gts match many
+ * dts; a gt with id 0 leaves dtMatches = 0; area bounds inclusive).  Writes every kept slot and npig (zeroed first). */
+int yl_cocoeval_evaluate(const yl_cocoeval_set* set, const yl_cocoeval_params* params, const yl_cocoeval_slots* out,
+                         void* stream);
+/* COCOeval.accumulate: one CTA per (category, area, maxDet, iouThr).  score[n_slots], rank[n_slots] and
+ * flags[A][T][n_slots] hold the slots of evaluate in accumulate order: category by category (category k owns
+ * [cat_slot_off[k], cat_slot_off[k+1])), each category's slots in np.argsort(-score, "mergesort") order over the
+ * image-ascending concatenation.  Writes precision[T][R][K][A][M], recall[T][K][A][M] and scores[T][R][K][A][M] (fp64,
+ * DEVICE), -1 where the category has no non-ignored gt; bit-identical to numpy. */
+int yl_cocoeval_accumulate(const yl_cocoeval_params* params, int n_cats, int n_slots, const int32_t* cat_slot_off,
+                           const double* score, const int32_t* rank, const uint8_t* flags, const int32_t* npig,
+                           double* precision, double* recall, double* scores, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -14,15 +14,16 @@ from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
 SOURCES = ["runtime.cu", "conv.cu", "conv_tc.cu", "conv_chain.cu", "dwpw_tc.cu", "conv_direct.cu", "layout.cu", "pool.cu", "attention.cu",
-           "decode.cu", "nms.cu", "preprocess.cu", "c3k2_fused.cu", "c3k2_tc.cu", "stem_fused.cu", "metrics.cu", "tta.cu", "embed.cu"]
+           "decode.cu", "nms.cu", "preprocess.cu", "c3k2_fused.cu", "c3k2_tc.cu", "stem_fused.cu", "metrics.cu", "tta.cu", "embed.cu",
+           "cocoeval.cu"]
 HEADERS = [HERE / "common.cuh", HERE / "conv_tc.cuh", HERE.parents[1] / "include" / "yl11.h"]
 OUT_DIR = HERE.parent / "yololite" / "lib"
 LIB = OUT_DIR / "libyl11.so"
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "--use_fast_math", "-Xptxas", "-v"]
 # nms.cu and decode.cu need IEEE arithmetic (bit-exact IoU / accurate expf), tta.cu ATen's bilinear arithmetic, embed.cu
-# keeps denormal activations in its sums: no fast-math
-NO_FAST_MATH = {"nms.cu", "decode.cu", "preprocess.cu", "metrics.cu", "tta.cu", "embed.cu"}
+# keeps denormal activations in its sums, cocoeval.cu is bit-exact fp64 against numpy: no fast-math
+NO_FAST_MATH = {"nms.cu", "decode.cu", "preprocess.cu", "metrics.cu", "tta.cu", "embed.cu", "cocoeval.cu"}
 
 
 def _nvcc():

@@ -131,6 +131,27 @@ class EmbedTap(C.Structure):
     _fields_ = [("x", Tensor), ("col", C.c_int32), ("_pad", C.c_int32)]
 
 
+class CocoevalSet(C.Structure):
+    """Mirror of `yl_cocoeval_set`."""
+
+    _fields_ = [(k, C.c_int32) for k in ("n_pairs", "n_cats", "n_slots", "max_gt", "max_dt")] + [
+        (k, C.c_void_p) for k in ("pair_cat", "gt_off", "gt_bbox", "gt_area", "gt_iscrowd", "gt_id", "slot_off", "dt_bbox",
+                                  "dt_score", "dt_area", "dt_id")]
+
+
+class CocoevalParams(C.Structure):
+    """Mirror of `yl_cocoeval_params`."""
+
+    _fields_ = [(k, C.c_void_p) for k in ("iou_thrs", "rec_thrs", "area_rng", "max_dets")] + [
+        (k, C.c_int32) for k in ("T", "R", "A", "M")]
+
+
+class CocoevalSlots(C.Structure):
+    """Mirror of `yl_cocoeval_slots`."""
+
+    _fields_ = [(k, C.c_void_p) for k in ("key", "rank", "flags", "npig")]
+
+
 _PROTOTYPES = {
     "yl_version": (C.c_int, []),
     "yl_last_error_string": (C.c_char_p, []),
@@ -206,6 +227,9 @@ _PROTOTYPES = {
     "yl_tta_merge": (C.c_int, [C.POINTER(TtaPass), C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "yl_embed_pool": (C.c_int, [C.POINTER(EmbedTap), C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                 C.POINTER(C.c_size_t), C.c_void_p]),
+    "yl_cocoeval_evaluate": (C.c_int, [C.POINTER(CocoevalSet), C.POINTER(CocoevalParams), C.POINTER(CocoevalSlots),
+                                       C.c_void_p]),
+    "yl_cocoeval_accumulate": (C.c_int, [C.POINTER(CocoevalParams), C.c_int, C.c_int] + [C.c_void_p] * 9),
 }
 
 EXPORTS = tuple(_PROTOTYPES)

@@ -40,6 +40,19 @@ _BOOL = {"half", "dnn", "rect", "agnostic_nms", "augment", "visualize", "save", 
          "save_json", "save_hybrid", "show", "verbose", "plots", "single_cls", "stream_buffer"}
 
 
+def get_save_dir(args) -> Path:
+    """Output directory of a run (reference cfg/__init__.py get_save_dir): `<project or runs/<task>>/<name or mode>`,
+    numbered `val2`, `val3`, ... when it exists, unless `exist_ok`.  Not created here."""
+    path = Path(args.project or Path("runs") / args.task) / (args.name or f"{args.mode}")
+    if path.exists() and not args.exist_ok:
+        for n in range(2, 9999):
+            p = Path(f"{path}{n}")
+            if not p.exists():
+                break
+        path = p
+    return path
+
+
 def get_cfg(cfg=DEFAULT_CFG, overrides=None) -> SimpleNamespace:
     """Merge `overrides` into the defaults with the reference's type/range checks."""
     base = dict(vars(cfg)) if isinstance(cfg, SimpleNamespace) else dict(cfg or DEFAULT_CFG_DICT)

@@ -84,6 +84,10 @@ class RectValLoader:
         files = sorted(str(p) for p in img_dir.rglob("*.*") if p.suffix[1:].lower() in IMG_FORMATS)
         if not files:
             raise FileNotFoundError(f"no images under {img_dir}")
+        return cls.from_files(files, label_dir, **kw)
+
+    @classmethod
+    def from_files(cls, files, label_dir=None, **kw):
         if label_dir is None:   # reference img2label_paths: .../images/... -> .../labels/...
             lab = [Path(f.replace("/images/", "/labels/", 1)).with_suffix(".txt") for f in files]
         else:
@@ -152,18 +156,32 @@ class RectValLoader:
             }
 
 
-def build_val_loader(data, imgsz=640, batch_size=16, stride=32, split="val"):
-    """`data`: a dataset yaml (keys path / val / names like coco8.yaml; `path` must resolve) or an image directory."""
+def load_data_yaml(data) -> dict:
+    """A dataset yaml (keys path / val / names like coco8.yaml) with `path` resolved against the yaml's directory."""
     from ..utils import yaml_load
 
     p = Path(str(data))
+    d = yaml_load(p)
+    root = Path(d.get("path") or p.parent)
+    d["path"] = root if root.is_absolute() else (p.parent / root).resolve()
+    return d
+
+
+def build_val_loader(data, imgsz=640, batch_size=16, stride=32, split="val"):
+    """`data`: a dataset yaml (keys path / val / names like coco8.yaml; `path` must resolve) or an image directory.  The
+    split is an image directory or, as in coco.yaml (`val: val2017.txt`), a `.txt` list of image paths relative to
+    `path`; labels are found by the `/images/` -> `/labels/` rule either way."""
+    p = Path(str(data))
+    kw = dict(imgsz=imgsz, batch_size=batch_size, stride=stride)
     if p.suffix in {".yaml", ".yml"}:
-        d = yaml_load(p)
-        root = Path(d.get("path") or p.parent)
-        if not root.is_absolute():
-            root = (p.parent / root).resolve()
-        img_dir = root / d[split]
-        names = d.get("names")
+        d = load_data_yaml(p)
+        split_path, names = d["path"] / d[split], d.get("names")
+        if split_path.suffix == ".txt":
+            lines = [x.strip() for x in split_path.read_text().splitlines() if x.strip()]
+            files = sorted(str(d["path"] / x) for x in lines if x.split(".")[-1].lower() in IMG_FORMATS)
+            if not files:
+                raise FileNotFoundError(f"no images listed in {split_path}")
+            return RectValLoader.from_files(files, **kw), names
     else:
-        img_dir, names = p, None
-    return RectValLoader.from_dirs(img_dir, imgsz=imgsz, batch_size=batch_size, stride=stride), names
+        split_path, names = p, None
+    return RectValLoader.from_dirs(split_path, **kw), names
