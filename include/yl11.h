@@ -161,6 +161,10 @@ typedef struct yl_conv_tc_plan {
     int tile_w, tile_h, tile_n;   /* A-tile box; tile_n > 1 = the same window of consecutive images stacked */
     int m_tiles, n_tiles;   /* n_tiles == 2 with co <= 256: the wave-quantisation N split */
     int co_tile, kblk, stages, grid, smem_bytes, tmem_cols;
+    int cw;                 /* TMEM columns per epilogue chunk (16 or 32) */
+    int stg_sub;            /* chunks per staged TMA store (2: 128-byte bf16 pixel rows) */
+    int epi_kind;           /* epilogue instantiation: 0-3 bf16 (SiLU?, residual?), 4 / 5 / 6 Detect box / class /
+                               class filter, 7 generic (f32 out, 16-column chunks, stored Detect raw map) */
 } yl_conv_tc_plan;
 int yl_conv_tc_info(const yl_conv_args* a, yl_conv_tc_plan* out);
 

@@ -7,6 +7,8 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+import test_conv_tc_paths_gpu as P
+
 pytestmark = pytest.mark.gpu
 
 
@@ -58,6 +60,34 @@ CONV_CASES = [
     (32, 32, 1, 1, 5, 23, 17, True, True, False, 0, 0, False, "k1_flat_ragged_tail_res"),
     (128, 256, 3, 1, 2, 20, 20, True, False, False, 0, 0, False, "k3_co256_long_k"),
 ]
+
+# the tcgen05 dispatch paths (test_conv_tc_paths_gpu.conv_paths) each case takes on a 148-SM B200
+TC_PATHS = {
+    "k1_sw128": {"epi0", "flat", "small_split"},
+    "k1_sw64": {"epi0", "flat", "small_split"},
+    "k1_sw32": {"epi0", "flat", "resident_weights"},
+    "k1_ci48_slices": {"epi0", "flat", "small_split"},
+    "k1_ci384_co256": {"epi0", "flat", "small_split"},
+    "k1_co512_two_ntiles": {"epi0", "flat", "small_split"},
+    "k1_co80_f32_bias_slice": {"epi7", "flat", "resident_weights", "f32_out"},
+    "k1_residual_noact": {"epi3", "flat", "small_split"},
+    "k3_s1": {"epi0", "patch_1cta", "patch_kblk64"},
+    "k3_co8": {"cw16", "epi7", "patch_2cta", "patch_kblk16"},
+    "k3_ci8_res_slice": {"cw16", "epi7", "patch_2cta", "patch_kblk16"},
+    "k3_residual": {"epi1", "image_stack", "resident_weights"},
+    "k3_ragged21": {"epi0", "small_split"},
+    "k3_12x20": {"epi0", "patch_1cta", "patch_kblk64"},
+    "k3_s2_sw32": {"epi0", "image_stack", "resident_weights", "stride2"},
+    "k3_s2_slice_in": {"epi0", "small_split", "stride2"},
+    "k3_s2_co256": {"epi0", "small_split", "stride2"},
+    "k1_upsample_into_concat": {"epi0", "small_split", "upsample"},
+    "k3_upsample": {"epi0", "small_split", "upsample"},
+    "k1_co48_chunk_tail": {"epi0", "flat", "resident_weights"},
+    "k1_co144_f32_multichunk": {"epi7", "flat", "resident_weights", "f32_out"},
+    "k3_20x20_stacked_images_res": {"epi1", "image_stack", "small_split"},
+    "k1_flat_ragged_tail_res": {"epi1", "flat", "resident_weights"},
+    "k3_co256_long_k": {"epi0", "image_stack", "small_split"},
+}
 
 DUAL_CASES = [
     # ci, co, k, s, n, h, w, y_pad, up_pad, tag
@@ -141,11 +171,22 @@ def test_conv_bn_act(ops, case, impl):
     supported = bool(_C.load().yl_conv_tc_supported(a))
     if impl == "tc":
         assert supported, "case expected to run on the tcgen05 path"
+        sms = torch.cuda.get_device_properties(0).multi_processor_count
+        reached = P.conv_paths(P.plan_info(a), n, ho, wo, co, sms, res=res, f32=f32out, up=up, stride=s)
+        assert sms != 148 or TC_PATHS[tag] <= reached, (tag, sorted(TC_PATHS[tag] - reached))
     ops.conv(xv, yv, pc, s, act, rv, up, impl=_C.IMPL_TCGEN05 if impl == "tc" else _C.IMPL_DIRECT)
     torch.cuda.synchronize()
     got = yv.torch_nhwc().float().cpu().permute(0, 3, 1, 2)
-    tol = 1e-3 if f32out else 2e-2
-    np.testing.assert_allclose(got.numpy(), ref.numpy(), rtol=tol, atol=tol)
+    if impl == "tc":
+        # fp64 of the operands the kernel reads (packed weights and bias, bf16 input and residual), per-element bound
+        w64, b64 = P.unpack_weights(pc)
+        res64 = rv.torch_nhwc().cpu().double().permute(0, 3, 1, 2) if res else None
+        ref64, pre, sabs = P.conv_reference(xv.torch_nhwc().cpu().double().permute(0, 3, 1, 2), w64, b64, s, act, res64,
+                                            up)
+        P.assert_within(got.double(), ref64, P.conv_bound(ref64, pre, sabs, not f32out, act), tag)
+    else:
+        tol = 1e-3 if f32out else 2e-2
+        np.testing.assert_allclose(got.numpy(), ref.numpy(), rtol=tol, atol=tol)
     # untouched channels of the destination buffer keep their fill value (slice write discipline)
     if y_pad:
         rest = torch.cat([yb[..., : y_pad // 2], yb[..., y_pad // 2 + co:]], -1)

@@ -180,19 +180,37 @@ def test_fused_decode_matches_decode_kernel_and_engine_path(golden):
     """The Detect decode fused into the head convs' epilogue (a) equals the standalone decode kernel fed by the
     raw maps within fp32 rounding of the fast exp, (b) is identical with and without materialising the raw maps
     (engine path `infer(want_raw=False)`), also for a batch that leaves the last 128-pixel tile ragged."""
+    _check_fused_decode(golden, "yolo11n", 80)
+
+
+@pytest.mark.parametrize("cfg,nc", [("yolo11n", 64), ("yolo11s", 256)])
+def test_fused_decode_matches_decode_kernel_and_engine_path_class_counts(golden, cfg, nc):
+    """The same parity for class counts at which a plain conv of these small class maps would be split into N tiles
+    (nc % 64 == 0): the fused class decode addresses its rows by the chunk index inside one N tile, so those convs must
+    run unsplit (nc = 256 on yolo11s: yolo11n's class branch would be 100 channels wide, which the fused decode does not
+    take)."""
+    _check_fused_decode(golden, cfg, nc)
+
+
+def _check_fused_decode(golden, cfg, nc):
+    from oracle.weights import tensor_for
     from yololite.nn.modules import Detect
     from yololite.nn.tasks import DetectionModel
 
     g = golden("model_yolo11n.npz")
     sd = model_state_dict(g)
+    if nc != 80:
+        shapes = DetectionModel(f"{cfg}.yaml", nc=nc, verbose=False).state_dict()
+        sd = {k: tensor_for(k, tuple(v.shape)) for k, v in shapes.items()}
     x = torch.rand(3, 3, 96, 160, generator=torch.Generator().manual_seed(5)).cuda()   # P5 map: 3*3*5 = 45 pixels
     outs = {}
     for fuse in (True, False):
         Detect.fuse_decode = fuse
         try:
-            m = DetectionModel("yolo11n.yaml", verbose=False)
+            m = DetectionModel(f"{cfg}.yaml", nc=nc, verbose=False)
             m.load_state_dict(sd)
             m = m.cuda().eval()
+            assert m.model[-1]._fuses_decode() == fuse
             y, raw = m(x)
             outs[fuse] = (y.cpu().numpy(), [r.cpu().numpy() for r in raw])
             if fuse:

@@ -629,12 +629,15 @@ int plan_conv_tc(const yl_conv_args* a, ConvTcParams& p, int* grid_out, size_t* 
     // second wave runs almost alone; halving the tile (2 CTAs/SM, 256 columns each) keeps every tile resident at once.
     {
         const long long m_est = ceil_div64((long long)x.n * Ho * Wo, 128);
-        // (the class-filter epilogue needs every class of a pixel in ONE tile)
+        // (a Detect epilogue runs as one N tile, see below)
         if (!chain && n_tiles == 1 && co16 > 128 && m_est > g_num_sms && m_est <= 2ll * g_num_sms && g_knobs.nsplit &&
-            a->det.mode != YL_DET_CLS_FILTER)
+            !a->det.pred)
             n_tiles = 2;
     }
-    p.co_tile = ceil_div(ceil_div(co16, n_tiles), 16) * 16;
+    // The epilogue drains and stores whole cw-column chunks (32 whenever n_tiles > 1), so every N tile but the last must
+    // be a multiple of 32 wide: a tile ending mid-chunk (co 144 as two 80-wide tiles) would store its out-of-tile
+    // accumulator columns over the first channels of the next tile.
+    p.co_tile = n_tiles > 1 ? ceil_div(ceil_div(co16, n_tiles), 32) * 32 : co16;
 
     // halo-patch mode: 3x3 stride-1 convs on thin inputs are L2->SM bound when every tap is fetched separately
     // (9 narrow TMA boxes per tile); fetch the (TH+2) x (TW+2) patch once instead and slide the A descriptor
@@ -651,7 +654,7 @@ int plan_conv_tc(const yl_conv_args* a, ConvTcParams& p, int* grid_out, size_t* 
     // Small problems (bs = 1 latency): with far fewer 128-pixel tiles than SMs a CTA's epilogue walks its N / 32 column
     // chunks serially (~0.45 us each, tools/timeline.py) while most of the GPU idles.  Split N down to 32-column tiles:
     // the chunks become parallel CTAs (the A tile is re-read from L2 by each, which is free at this size).
-    if (!chain && !patch && g_knobs.small_nsplit && (a->det.mode == YL_DET_NONE || a->det.mode == YL_DET_CLS)) {
+    if (!chain && !patch && g_knobs.small_nsplit && !a->det.pred) {
         const long long m_est = ceil_div64((long long)x.n * Ho * Wo, 128);
         int nt = n_tiles;
         while (m_est * nt * 2 <= g_num_sms && co16 % (64 * nt) == 0 && co16 / (2 * nt) >= 32) nt *= 2;
@@ -660,6 +663,12 @@ int plan_conv_tc(const yl_conv_args* a, ConvTcParams& p, int* grid_out, size_t* 
             p.co_tile = co16 / nt;
         }
     }
+    // Detect epilogues take every channel of a pixel in ONE N tile: the box decode (four DFL sides) and the class filter
+    // (running best class) keep per-pixel state across the chunks, and the decode addresses prediction rows by the chunk
+    // index inside the tile.  (Splitting the class conv would only help nc % 64 == 0 or nc > 128 at small batches; a
+    // tile-aware decode measured ~0.2 % slower at bs = 64 on a B200 at 1000 W: it changes the register allocation of the
+    // whole production kernel.)
+    YL_CHECK(n_tiles == 1 || !a->det.pred, YL_ERR_UNSUPPORTED, "a Detect epilogue needs one N tile (got %d)", n_tiles);
     const CUtensorMapSwizzle swp = swizzle_for_bytes(p.kblk * 2);
 
     // M tiling + activation tensor maps
@@ -1038,6 +1047,9 @@ int conv_tc_info(const yl_conv_args* a, yl_conv_tc_plan* out) {
     out->grid = grid;
     out->smem_bytes = (int)smem;
     out->tmem_cols = (int)p.tmem_cols;
+    out->cw = p.cw;
+    out->stg_sub = p.stg_sub;
+    out->epi_kind = p.epi_kind;
     return YL_OK;
 }
 

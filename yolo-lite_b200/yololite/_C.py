@@ -102,7 +102,8 @@ class ConvTcPlan(C.Structure):
     """Mirror of `yl_conv_tc_plan` (how the tcgen05 path would run a conv; yl_conv_tc_info)."""
 
     _fields_ = [(k, C.c_int32) for k in ("flat", "patch", "wres", "tile_w", "tile_h", "tile_n", "m_tiles", "n_tiles",
-                                         "co_tile", "kblk", "stages", "grid", "smem_bytes", "tmem_cols")]
+                                         "co_tile", "kblk", "stages", "grid", "smem_bytes", "tmem_cols", "cw",
+                                         "stg_sub", "epi_kind")]
 
 
 class ConvChain(C.Structure):
